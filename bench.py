@@ -78,6 +78,8 @@ def parse():
     ap.add_argument("--ref-seconds", type=float, default=20.0, help="timed window of the cpu_baseline leg (one core), seconds")
     ap.add_argument("--ref-window", type=float, default=60.0, help="timed window of --impl reference (every core), seconds")
     ap.add_argument("--ref-test-sims", type=int, default=0, help="smoke tests only: sims/move of the reference worker")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what they computed as DIR/<name>.npy "
+                    "(float32, at most 60 MB; rank 0), to compare two builds output for output")
     args = ap.parse_args()
     select_workload(args.workload)
     if args.workload == "go9":          # smaller defaults: a Go 9x9 tree slab is 6.5 MB, a sample row 5.8 KB
@@ -266,6 +268,8 @@ def run_ours(args):
         st = eng.stats()
         playing, failed = eng.poll()
         assert failed == 0 and playing == args.slots, (playing, failed)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, eng)
 
         # ---- roofline leg: the search launch alone, timed with events on its stream
         n_probe = 64
@@ -384,6 +388,46 @@ def run_ours(args):
         emit(result)
 
 
+DUMP_BYTES_PER_GROUP = 30 * 10**6      # two groups of arrays: --dump-outputs writes at most 60 MB
+
+
+def dump_outputs(out_dir, eng):
+    """--dump-outputs: what the timed steps computed, as float32 .npy files, for comparing two builds on identical inputs.
+    eval_inputs / eval_logits / eval_values: the leaf batch of the last round and the network's outputs for it.  The
+    search kernel hands out batch rows in no fixed order, so the rows are sorted by their bytes.
+    samples_states / samples_distributions / samples_outcomes: the sample rows of every game finished so far, in the
+    reference's order (games, moves, symmetries).  A group larger than DUMP_BYTES_PER_GROUP keeps a fixed, seeded
+    sample of its rows, in order."""
+    import numpy as np
+    import torch
+    nn = eng._nn
+    torch.cuda.synchronize(nn["dev"])
+
+    def keep(n, row_bytes):
+        cap = DUMP_BYTES_PER_GROUP // row_bytes
+        return np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+    class Counter:                 # __cuda_array_interface__ over the device count of rows the last launch queued
+        __cuda_array_interface__ = dict(shape=(1,), typestr="<i4", data=(nn["rows"], False), version=3, strides=None, stream=None)
+    rows = int(torch.as_tensor(Counter(), device=nn["dev"]).item())
+    x = nn["inp"][:rows].reshape(rows, -1).cpu().numpy()
+    logits = nn["logits"][:rows].cpu().numpy()
+    flat = np.ascontiguousarray(np.concatenate([x, logits, nn["value"][:rows].cpu().numpy().reshape(rows, 1)], 1))
+    flat = flat[np.argsort(flat.view(np.dtype((np.void, flat.shape[1] * 4))).ravel(), kind="stable")]
+    flat = flat[keep(rows, flat.shape[1] * 4)]
+    P, A = x.shape[1], logits.shape[1]
+    out = {"eval_inputs": flat[:, :P].reshape((-1,) + tuple(nn["inp"].shape[1:])), "eval_logits": flat[:, P:P + A],
+           "eval_values": flat[:, P + A]}
+
+    states, dists, outcomes = eng.collect_samples_device()
+    idx = torch.from_numpy(keep(states.shape[0], 4 * (int(np.prod(states.shape[1:])) + dists.shape[1] + 1))).to(states.device)
+    out.update(samples_states=states[idx], samples_distributions=dists[idx], samples_outcomes=outcomes[idx])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 def run_e2e(args, local, module, flat_params, weight_bytes, barrier, evalnet, rank=0, world=1):
     """Full generations through the public API with host buffers.  Every e2e step is one generation as SURVEY.md 8(d)
     config 4 / 8(e) describe it: rank 0 holds the new network's weights in host memory and broadcasts the flat parameter +
@@ -486,10 +530,18 @@ def cpu_baseline(args, threads, seconds, game="othello"):
     CPU), `threads` single-threaded processes (one per host core, the reference's deployment model).  Protocol of
     BASELINE.md section 3: every process plays one discarded warm-up game, then full games through the reference's own
     SPRL::runIteration until `seconds` of wall time have passed (the game in progress is finished and counted)."""
-    if not os.path.exists(ref_worker_path()):
-        return cpu_baseline_port(seconds)
-    model = traced_model_file()
     sims = args.ref_test_sims or SIMS
+    if not os.path.exists(ref_worker_path()):
+        r = cpu_baseline_port(sims, seconds)
+    else:
+        r = cpu_baseline_reference(threads, seconds, game, sims)
+    if args.ref_test_sims:
+        r["test_override"] = f"{sims} sims/move instead of {SIMS} (smoke test of the arm, not a measurement)"
+    return r
+
+
+def cpu_baseline_reference(threads, seconds, game, sims):
+    model = traced_model_file()
     t0 = time.time()
     procs = [subprocess.Popen([ref_worker_path(), game, model, "0", str(100000 * (i + 1)), str(sims), str(MAX_BATCH), str(MAX_QUEUE),
                                str(EPS), str(ALPHA), str(seconds)], stdout=subprocess.PIPE, text=True) for i in range(threads)]
@@ -507,13 +559,12 @@ def cpu_baseline(args, threads, seconds, game="othello"):
                    f"game(s) through the reference's runIteration in a {window:.1f} s window, {sims} sims/move, traced 2x64 net on CPU "
                    f"(LibTorch, 1 thread each); {wall:.1f} s wall in all",
          "cpu": cpu_model(), "host_cores": os.cpu_count()}
-    if args.ref_test_sims:
-        r["test_override"] = f"{sims} sims/move instead of {SIMS} (smoke test of the arm, not a measurement)"
     return r
 
 
-def cpu_baseline_port(seconds):
-    """Fallback when oracle/_ref was not built: the plain-C oracle port, one thread."""
+def cpu_baseline_port(sims, seconds):
+    """Fallback when oracle/_ref was not built: the plain-C oracle port, one thread, full games at `sims` sims/move until
+    `seconds` of wall time have passed (the game in progress is finished and counted)."""
     import numpy as np
     import torch
     sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -527,11 +578,25 @@ def cpu_baseline_port(seconds):
             lg, v = net(torch.from_numpy(np.array(x)))
         return lg.numpy(), v.numpy().reshape(-1)
 
+    def play(game):
+        return O.selfplay(O.OG_OTHELLO, O.OE_CALLBACK, 0, game, 1, sims, MAX_BATCH, MAX_QUEUE, EPS, ALPHA, eval_fn=fn)
+
+    play(0)                     # discarded warm-up game, as in the reference protocol
+    games = moves = sims_done = 0
     t0 = time.time()
-    r = O.selfplay(O.OG_OTHELLO, O.OE_CALLBACK, 0, 0, 1, 100, MAX_BATCH, MAX_QUEUE, EPS, ALPHA, eval_fn=fn)
-    dt = time.time() - t0
-    return {"value": round(r["stats"]["total_traversals"] / dt, 1), "unit": "sims/s", "cores": 1, "kind": "port",
-            "sample": "1 game at 100 sims/move through the C oracle with the network on CPU via a Python callback"}
+    while True:
+        r = play(1 + games)
+        games += 1
+        moves += int(r["game_moves"].sum())
+        sims_done += r["stats"]["total_traversals"]
+        dt = time.time() - t0
+        if dt >= seconds:
+            break
+    return {"value": round(sims_done / dt, 1), "unit": "sims/s", "cores": 1, "kind": "port",
+            "moves_per_sec": round(moves / dt, 2), "window_seconds": round(dt, 2), "games": games,
+            "sims_per_move": round(sims_done / moves, 2),
+            "sample": f"one discarded warm-up game, then {games} full game(s) at {sims} sims/move through the C oracle with "
+                      f"the network on CPU via a Python callback, one thread, in a {dt:.1f} s window"}
 
 
 def cpu_model():
