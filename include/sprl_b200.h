@@ -298,7 +298,10 @@ int sprl_write_npy_f32(const char* path, const float* h_data, const uint64_t* sh
  * tcgen05 kernel for boards up to 8x8 (Othello, Go 7x7, Connect Four: two boards per MMA tile) and up
  * to 128 cells in rows of at most 16 (Go 9x9: one board per tile): conv tower on the tensor cores with
  * a two-term fp16 split (fp32-level accuracy, fp32 accumulate), BatchNorm folded, head FCs in a second
- * kernel.  Other shapes keep using the traced module through sprl_forward_fn. */
+ * kernel.  The head FCs stage their weights and a 64-board step of head activations in shared memory, which
+ * caps boards with two policy channels at 87 cells (Go 9x9's 81 fit); with one policy channel the whole
+ * 128 cells fit.  Limits: 1 to 21 input planes, 0 to 7 residual blocks of 64 channels, 1 or 2 policy channels,
+ * 1 to 84 actions.  Other shapes keep using the traced module through sprl_forward_fn. */
 typedef struct {
     const float *weight, *bias;                             /* conv: [out, in, 3, 3], [out] */
     const float *bn_weight, *bn_bias, *bn_mean, *bn_var;    /* BatchNorm2d affine + running stats, [out] */
@@ -320,8 +323,9 @@ typedef struct {
 typedef struct sprl_evalnet sprl_evalnet;
 
 int sprl_evalnet_create(int device, const sprl_network_params* h_params, sprl_evalnet** out);
-/* New generation's weights, same shape: overwritten in place (device addresses stay valid
- * for captured CUDA graphs). */
+/* New generation's weights, same shape: overwritten in place.  Device addresses stay valid, and the per-layer
+ * weight scales live in device memory too, so a CUDA graph captured before the update replays with the new
+ * weights and their scales. */
 int sprl_evalnet_update(sprl_evalnet* net, const sprl_network_params* h_params);
 /* INetwork::evaluate's forward (networks/GridNetwork.hpp:99-102) on device buffers:
  * d_in [batch, in_planes, rows, cols] -> d_logits [batch, actions], d_value [batch].  Asynchronous on
@@ -341,7 +345,8 @@ int sprl_evalnet_info(sprl_evalnet* net, int64_t* upload_bytes, int32_t* ring_st
  * when a block fits, else the streaming kernel (weights re-read from L2 per tile).  Both accumulate the conv tower in
  * the same order; the resident kernel computes the 1x1 head convolutions as fp32 FMAs instead of split-fp16 MMAs, so
  * their outputs agree to rounding (1e-6), each within 2e-6 of the fp64 forward.  STREAMING / RESIDENT force one of
- * them (tests, A/B timing). */
+ * them (tests, A/B timing).  The choice applies to forwards enqueued after the call: a captured CUDA graph keeps
+ * replaying the kernel it was captured with. */
 #define SPRL_EVALNET_PATH_AUTO 0
 #define SPRL_EVALNET_PATH_STREAMING 1
 #define SPRL_EVALNET_PATH_RESIDENT 2
@@ -351,7 +356,8 @@ int sprl_evalnet_set_path(sprl_evalnet* net, int path);
  * the fp64 forward, the accuracy of the reference's fp32 LibTorch path.  FP16 (opt-in, resident kernel only): the hi
  * terms alone, one MMA per product, fp32 accumulation, fp32 bias / residual / head layers -- the "bf16/fp16 with fp32
  * accumulate" design point of an inference-only evaluator; about 1e-3 on logits.  It is NOT the reference's precision:
- * self-play statistics differ from an fp32 evaluator's, and a throughput measured with it is a different metric. */
+ * self-play statistics differ from an fp32 evaluator's, and a throughput measured with it is a different metric.
+ * The mode applies to forwards enqueued after the call: a captured CUDA graph keeps the mode it was captured with. */
 #define SPRL_EVALNET_PRECISION_FP32_SPLIT 0
 #define SPRL_EVALNET_PRECISION_FP16 1
 int sprl_evalnet_set_precision(sprl_evalnet* net, int precision);

@@ -146,7 +146,8 @@ struct NetDev {
     int nst;                 // ring stages
     float* head_act;         // [batch][(policy_channels + 1) * 64]: ReLU'd 1x1-conv head activations, consumed by k_heads
     unsigned long long* error_flag;   // [0] pipeline barrier time-out, [1] an activation left the fp16-split range
-    float inv_scale[MAX_LAYERS];      // 2^-(ACT_SHIFT + weight shift of the layer): accumulator -> real units
+    const float* inv_scale;  // [MAX_LAYERS] 2^-(ACT_SHIFT + weight shift of the layer): accumulator -> real units.  In device
+                             // memory, not in this by-value struct: a captured CUDA graph must see the scales of update()
     long long* timing;       // [grid][12] cycle counters per role (debug >= 0: always written, tiny)
     int single_pass;         // SPRL_EVALNET_PRECISION_FP16 (resident kernel): one fp16 MMA per product instead of the three of the hi/lo split
     long long* trace;        // -DSPRL_EVALNET_TRACE builds: [phase][role: mma, epilogue X, epilogue Y][1 + 255 events] of CTA 0, clock << 12 | code
@@ -624,13 +625,14 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
 #ifndef SPRL_EVALNET_NO_PREFETCH
                 if (layer == n_layers - 1 && tile + gridDim.x < tile_end) load_planes(tile + gridDim.x, half, vnext);
 #endif
+                // accumulator -> image units for the conv layers (real units for the heads); exact powers of two (read
+                // before the wait below, which hides the load)
+                const float inv_scale = __ldg(net.inv_scale + layer) * (layer < n_layers - 1 ? ACT_SCALE : 1.0f);
                 { long long a = NOW(); mbar_wait(bar_acc, acc_phase, net.error_flag, 3); t_acc += NOW() - a; }
                 const long long t_layer = NOW();
                 acc_phase ^= 1u;
                 tc_fence_after();
                 const float* bias = s_bias + layer * CH;
-                // accumulator -> image units for the conv layers (real units for the heads); exact powers of two
-                const float inv_scale = net.inv_scale[layer] * (layer < n_layers - 1 ? ACT_SCALE : 1.0f);
                 if (layer < n_layers - 1 && net.debug >= 5) {
                     // timing experiment: no epilogue work
                 } else if (layer < n_layers - 1) {
@@ -982,7 +984,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
     const int in_k = KSTEP_CH * ((3 * P + KSTEP_CH - 1) / KSTEP_CH);      // stem input channels: (dy, plane), see k_evalnet
     const double eps = p->bn_eps > 0 ? p->bn_eps : 1e-5;
     std::vector<unsigned short> units;
-    std::vector<float> bias((size_t)L * C, 0.0f);
+    std::vector<float> bias((size_t)L * C, 0.0f), inv_scale(MAX_LAYERS, 0.0f);
     struct LayerW { std::vector<std::vector<float>> b; int n_pad, kk, shift; };       // b[dy * ndx + dx][n * kk + k], kept for the resident format
     std::vector<LayerW> layers;
     auto conv_layer = [&](const sprl_conv_bn_params& c, int cin, int kk, int layer) {
@@ -997,7 +999,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
                 for (int ci = 0; ci < cin; ++ci)
                     b[t][(size_t)co * kk + ci] = (float)((double)c.weight[((size_t)co * cin + ci) * 9 + t] * scale[co]);
         const int shift = weight_shift(b);
-        e->dev.inv_scale[layer] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
+        inv_scale[layer] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
         for (int dy = 0; dy < 3; ++dy)
             append_units(units, std::vector<std::vector<float>>(b.begin() + 3 * dy, b.begin() + 3 * dy + 3), C, kk, shift);
         layers.push_back(LayerW{ std::move(b), C, kk, shift });
@@ -1014,7 +1016,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
                         b[dx][(size_t)co * in_k + dy * P + ci] = (float)((double)c.weight[((size_t)co * P + ci) * 9 + dy * 3 + dx] * scale);
         }
         const int shift = weight_shift(b);
-        e->dev.inv_scale[0] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
+        inv_scale[0] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
         append_units(units, b, C, in_k, shift);
         layers.push_back(LayerW{ std::move(b), C, in_k, shift });
     }
@@ -1030,7 +1032,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
         for (int ci = 0; ci < C; ++ci) b[(size_t)pc * C + ci] = p->value_conv_w[ci];
         bias[(size_t)(L - 1) * C + pc] = p->value_conv_b[0];
         const int shift = weight_shift(bb);
-        e->dev.inv_scale[L - 1] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
+        inv_scale[L - 1] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
         append_units(units, bb, HEAD_N, C, shift);
         layers.push_back(LayerW{ std::move(bb), HEAD_N, C, shift });
     }
@@ -1142,6 +1144,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
     }
     if (!rc) e->phases = phases;
     if (!rc) rc = e->upload(bias, &e->dev.bias);
+    if (!rc) rc = e->upload(inv_scale, &e->dev.inv_scale);
     if (!rc) rc = e->upload(pfc_wt, &e->dev.pfc_wt);
     if (!rc) rc = e->upload(pfc_b, &e->dev.pfc_b);
     if (!rc) rc = e->upload(vfc1_wt, &e->dev.vfc1_wt);

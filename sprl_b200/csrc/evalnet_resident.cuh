@@ -290,6 +290,8 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
             for (int j = 0; j <= last_stage; ++j) {
                 const RbStage S = ph.st[j];
                 const bool feed = j == last_stage && has_next;       // this epilogue also writes the next tile's input
+                // accumulator -> image units; exact powers of two (read before the wait below, which hides the load)
+                const float inv_scale = __ldg(net.inv_scale + S.layer) * ACT_SCALE;
                 if (j == 0 && !planes_in && lane == 0 && next < n_tiles) {
                     // the next tile's activations towards L2, a whole tile ahead of their use
                     const float* nsrc = ph.act + (size_t)next * RB_ACT_TILE_FLOATS + (w8 & 3) * 32 * 4;
@@ -308,8 +310,6 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
                 // the image is free from here on in the last stage: its MMAs are complete and its output does not go there
                 if (feed && planes_in) put_planes(next);
                 const float* bias = s_bias + j * CH;
-                // accumulator -> image units; exact powers of two
-                const float inv_scale = net.inv_scale[S.layer] * ACT_SCALE;
                 float hp0 = 0.0f, hp1 = 0.0f, hp2 = 0.0f;            // head convolutions over this thread's 32 channels
 #pragma unroll 1
                 for (int q = 2 * half; q < 2 * half + 2; ++q) {
