@@ -298,10 +298,14 @@ int sprl_write_npy_f32(const char* path, const float* h_data, const uint64_t* sh
  * tcgen05 kernel for boards up to 8x8 (Othello, Go 7x7, Connect Four: two boards per MMA tile) and up
  * to 128 cells in rows of at most 16 (Go 9x9: one board per tile): conv tower on the tensor cores with
  * a two-term fp16 split (fp32-level accuracy, fp32 accumulate), BatchNorm folded, head FCs in a second
- * kernel.  The head FCs stage their weights and a 64-board step of head activations in shared memory, which
- * caps boards with two policy channels at 87 cells (Go 9x9's 81 fit); with one policy channel the whole
- * 128 cells fit.  Limits: 1 to 21 input planes, 0 to 7 residual blocks of 64 channels, 1 or 2 policy channels,
- * 1 to 84 actions.  Other shapes keep using the traced module through sprl_forward_fn. */
+ * kernel.  Limits: 1 to 21 input planes, 0 to 7 residual blocks of 64 or 128 channels, a value hidden layer as
+ * wide as the tower, 1 or 2 policy channels, 1 to 84 actions.  The head FCs stage their weights and a step of head
+ * activations in shared memory: with 64 channels a 64-board step, which caps boards with two policy channels at
+ * 87 cells (Go 9x9's 81 fit); with 128 channels a 32-board step, which caps them at 110 cells.  With one policy
+ * channel the whole 128 cells fit at both widths.  128-channel networks always run the streaming kernel (one CTA
+ * per SM; a layer's weights do not fit the resident kernel), so for them SPRL_EVALNET_PATH_RESIDENT and
+ * SPRL_EVALNET_PRECISION_FP16 fail with SPRL_E_STATE.  Other shapes keep using the traced module through
+ * sprl_forward_fn. */
 typedef struct {
     const float *weight, *bias;                             /* conv: [out, in, 3, 3], [out] */
     const float *bn_weight, *bn_bias, *bn_mean, *bn_var;    /* BatchNorm2d affine + running stats, [out] */
@@ -323,7 +327,7 @@ typedef struct {
 typedef struct sprl_evalnet sprl_evalnet;
 
 int sprl_evalnet_create(int device, const sprl_network_params* h_params, sprl_evalnet** out);
-/* New generation's weights, same shape: overwritten in place.  Device addresses stay valid, and the per-layer
+/* New generation's weights, same shape (a change of width is refused): overwritten in place.  Device addresses stay valid, and the per-layer
  * weight scales live in device memory too, so a CUDA graph captured before the update replays with the new
  * weights and their scales. */
 int sprl_evalnet_update(sprl_evalnet* net, const sprl_network_params* h_params);

@@ -48,6 +48,9 @@
 //     boards wider than 8 (Go 9x9) use the LINEAR lattice (k_evalnet<true>): one board per tile, cell
 //     r * cols + c = TMEM lane, vertical taps = descriptor shifts by `cols` slots, and the left / right
 //     neighbours that live in another warp are exchanged through a small shared-memory scratch.
+//   * 128-channel towers (k_evalnet<., 128>): every conv layer is two output halves of 64 channels, each the same N = 192
+//     MMA into its own accumulators; with the residual they take all 512 TMEM columns, so that instantiation runs one CTA
+//     per SM.  The resident kernel has no room for their weights: they always take this kernel.
 //   * A board's outputs do not depend on its row in the batch or on its tile partner (every CTA accumulates
 //     in the same order), and the batch size may be read on the device (d_rows): the search kernel hands leaf
 //     rows out by atomics and self-play stays reproducible.
@@ -65,7 +68,8 @@ namespace sprl {
 namespace evalnet {
 
 constexpr int TILE_M = 128;                  // cells per tile (two 8x8 boards)
-constexpr int CH = 64;                       // tower width
+constexpr int CH = 64;                       // tower width of the resident kernel and of the streaming kernel's output halves
+constexpr int WIDE_CH = 128;                 // the other tower width the streaming kernel runs: two output halves of CH
 constexpr int KCH = 8;                       // channels per 16-byte group (8 halfs)
 constexpr int NCG = CH / KCH;                // channel groups
 constexpr int KSTEP_CH = 2 * KCH;            // input channels per MMA (kind::f16: K = 16)
@@ -73,7 +77,6 @@ constexpr int ACT_SHIFT = 4;                 // activations are stored x 2^ACT_S
 constexpr float ACT_SCALE = 16.0f, HALF_MAX = 65504.0f;
 constexpr int SLOTS = 160;                   // 20 storage rows x 8 cells
 constexpr int CG_STRIDE = SLOTS * 16;        // bytes per channel group of the image
-constexpr int IMG_BYTES = NCG * CG_STRIDE;   // 20,480
 #ifndef SPRL_EVALNET_UNIT_KSTEPS
 #define SPRL_EVALNET_UNIT_KSTEPS 2
 #endif
@@ -112,30 +115,41 @@ constexpr int ROTATE = SPRL_EVALNET_ROTATE;
 constexpr bool PAIR = SPRL_EVALNET_PAIR != 0;
 static_assert(!PAIR || CLUSTER == 2, "the CTA pair is a cluster of two");
 constexpr int UNIT_SLOT = PAIR ? UNIT_BYTES / 2 : UNIT_BYTES;   // bytes of a ring stage in one CTA
-constexpr int TMEM_COLS = 256;               // [dx * 64 + channel] = Z_dx (all three split products); [192, 256) = residual
-constexpr int RES_COL = 3 * CH;              // the block input of the current residual block, fp32, one cell per lane
+constexpr int RES_COL = 3 * CH;              // resident kernel: the block input of the current residual block, fp32, one cell per lane
 #ifndef SPRL_EVALNET_CTAS_PER_SM
 #define SPRL_EVALNET_CTAS_PER_SM 2
 #endif
-constexpr int CTAS_PER_SM = SPRL_EVALNET_CTAS_PER_SM;   // resident CTAs per SM (each owns 256 TMEM columns)
-constexpr int MAX_SMEM = (232448 - (CTAS_PER_SM - 1) * 1024) / CTAS_PER_SM;   // 227 KB per SM, 1 KB reserved per extra CTA
 
-// shared memory map (bytes); the ring, the biases and the barriers follow at run-time offsets
-constexpr int OFF_AHI = 0;
-constexpr int OFF_ALO = OFF_AHI + IMG_BYTES;
-constexpr int OFF_RING = OFF_ALO + IMG_BYTES;                    // 81,920
+// Streaming kernel (k_evalnet) geometry of a tower of C channels.  The C outputs of a conv layer are C / 64 output
+// halves of 64 channels; every half is the same N = 192 MMA (3 dx x 64) into its own 192 TMEM columns
+// [half * 192 + dx * 64 + channel], and the residual follows them: 64 channels use 256 columns, so two CTAs share an
+// SM; 128 channels use all 512, so one CTA has the SM (its shared memory, 2 x 40 KB of image, holds ~5 ring stages).
+template <int C> struct Width {
+    static constexpr int NH = C / CH;                        // output halves
+    static constexpr int IMG_BYTES = (C / KCH) * CG_STRIDE;  // 20,480 / 40,960
+    static constexpr int TMEM_COLS = NH == 1 ? 256 : 512;
+    static constexpr int RES_COL = 3 * CH * NH;              // the block input of the current residual block, fp32, one cell per lane
+    static constexpr int CTAS_PER_SM = NH == 1 ? SPRL_EVALNET_CTAS_PER_SM : 1;   // resident CTAs per SM
+    static constexpr int MAX_SMEM = (232448 - (CTAS_PER_SM - 1) * 1024) / CTAS_PER_SM;   // 227 KB per SM, 1 KB reserved per extra CTA
+    static constexpr int CHUNKS = C / 32;                    // 16-channel epilogue chunks per warp (two warps per lane quarter)
+    // shared memory map (bytes); the ring, the biases and the barriers follow at run-time offsets
+    static constexpr int OFF_AHI = 0, OFF_ALO = IMG_BYTES, OFF_RING = 2 * IMG_BYTES;
+    // TMEM column of accumulator dx = -1 for channels [16 q, 16 q + 16); dx = 0 and +1 follow at +64 and +128
+    __device__ static constexpr int zcol(int q) { return q * 16 + (NH > 1 ? (q >> 2) * 2 * CH : 0); }
+};
+static_assert(Width<WIDE_CH>::RES_COL + WIDE_CH == Width<WIDE_CH>::TMEM_COLS, "128 channels fill the TMEM");
 
 struct NetDev {
     const unsigned short* wunits;   // packed fp16 weight units in consumption order, `replicas` copies back to back
     long long wunits_bytes;  // bytes of one copy
     int replicas;
-    const float* bias;       // [n_layers][64]
+    const float* bias;       // [n_layers][channels]
     const float* pfc_wt;     // [128][actions]  (policy_fc.weight transposed)
     const float* pfc_b;      // [actions]
-    const float* vfc1_wt;    // [64][64]        (value_fc1.weight transposed)
-    const float* vfc1_b;     // [64]
-    const float* vfc2_w;     // [64] weights, then the bias
-    const float* head_w;     // [4][64] fp32 weights of the 1x1 head convolutions (rows 0..pc-1 policy, row pc value, rest zero): k_evalnet_resident
+    const float* vfc1_wt;    // [cells][value_hidden] (value_fc1.weight transposed)
+    const float* vfc1_b;     // [value_hidden]
+    const float* vfc2_w;     // [value_hidden] weights, then the bias
+    const float* head_w;     // [4][channels] fp32 weights of the 1x1 head convolutions (rows 0..pc-1 policy, row pc value, rest zero): k_evalnet_resident
     int n_layers;            // 1 stem + 2*blocks + 1 heads
     int rows, cols;          // board: cell (r, c) lives at lattice position (r, c) of an 8 x 8 tile half, or ...
     int linear;              // ... boards wider or taller than 8 (Go 9x9): ONE board per tile, cell r * cols + c = TMEM lane
@@ -154,8 +168,8 @@ struct NetDev {
     int debug;               // timing experiments only (SPRL_EVALNET_DEBUG): 1 skip lo pass, 3 no MMAs, 5 = 3 + no conv epilogue, 6 = MMAs but no conv epilogue
 };
 
-__host__ __device__ inline int smem_bytes_for(int n_layers, int nst) {
-    return OFF_RING + nst * UNIT_SLOT + n_layers * CH * 4 + (3 * nst + 2) * 8 + 16 + XCH_BYTES;
+template <int C> inline int smem_bytes_for(int n_layers, int nst) {
+    return Width<C>::OFF_RING + nst * UNIT_SLOT + n_layers * C * 4 + (3 * nst + 2) * 8 + 16 + XCH_BYTES;
 }
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -351,13 +365,14 @@ __device__ __forceinline__ uint32_t instr_desc_f16(int m, int n) {
 // W_hi(dx=-1) | W_hi(0) | W_hi(+1) | W_lo(-1) | W_lo(0) | W_lo(+1), n rows each.  Per k-step three
 // MMAs with N = 3n accumulate into the same columns [dx*n + channel]: A_hi*[W_hi x3], A_hi*[W_lo x3]
 // and A_lo*[W_hi x3] -- each 4 KB read of A feeds 192 output columns.  The 1x1 head convolution is
-// the same with one dx.
-struct LayerGeom { int ndy, ndx, ksteps, n, units_per_dy; };
-__host__ __device__ inline LayerGeom layer_geom(int layer, int n_layers, int in_ksteps) {
+// the same with one dx.  A conv layer of 128 channels is two such layers of 64 outputs over the same
+// input, one after the other (`nh` output halves): all units of half 0, then all units of half 1.
+struct LayerGeom { int ndy, ndx, ksteps, n, units_per_dy, nh; };
+template <int C> __host__ __device__ inline LayerGeom layer_geom(int layer, int n_layers, int in_ksteps) {
     LayerGeom g;
-    if (layer == 0) { g.ndy = 1; g.ndx = 3; g.ksteps = in_ksteps; g.n = CH; }      // stem: the three dy taps are folded into K
-    else if (layer == n_layers - 1) { g.ndy = 1; g.ndx = 1; g.ksteps = CH / KSTEP_CH; g.n = HEAD_N; }
-    else { g.ndy = 3; g.ndx = 3; g.ksteps = CH / KSTEP_CH; g.n = CH; }
+    if (layer == 0) { g.ndy = 1; g.ndx = 3; g.ksteps = in_ksteps; g.n = CH; g.nh = C / CH; }      // stem: the three dy taps are folded into K
+    else if (layer == n_layers - 1) { g.ndy = 1; g.ndx = 1; g.ksteps = C / KSTEP_CH; g.n = HEAD_N; g.nh = 1; }
+    else { g.ndy = 3; g.ndx = 3; g.ksteps = C / KSTEP_CH; g.n = CH; g.nh = C / CH; }
     g.units_per_dy = (g.ksteps + UNIT_KS - 1) / UNIT_KS;
     return g;
 }
@@ -389,16 +404,17 @@ __device__ __forceinline__ int cell_slot(int m) { return m + 16; }
 #define TRACE_END() do { } while (0)
 #endif
 
-template <bool LINEAR>
-__global__ void __launch_bounds__(THREADS, CTAS_PER_SM)
+template <bool LINEAR, int C>
+__global__ void __launch_bounds__(THREADS, Width<C>::CTAS_PER_SM)
 k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsigned* __restrict__ d_rows,
           float* __restrict__ logits, float* __restrict__ value) {
+    using W = Width<C>;
     extern __shared__ __align__(128) unsigned char smem[];
     if (d_rows) batch = min((long long)*d_rows, batch);          // batch size decided on the device by the previous kernel
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_layers = net.n_layers, nst = net.nst;
     const uint32_t s_base = smem_u32(smem);
-    const int off_bias = OFF_RING + nst * UNIT_SLOT, off_bars = off_bias + n_layers * CH * 4, off_tmem = off_bars + (3 * nst + 2) * 8;
+    const int off_bias = W::OFF_RING + nst * UNIT_SLOT, off_bars = off_bias + n_layers * C * 4, off_tmem = off_bars + (3 * nst + 2) * 8;
     const uint32_t bar_full = s_base + off_bars, bar_empty = bar_full + nst * 8, bar_acc = bar_empty + nst * 8;
     const uint32_t bar_pfull = bar_acc + 8, bar_img = bar_pfull + nst * 8;      // pair mode, used in the leader: peer's half / image
     float* s_bias = reinterpret_cast<float*>(smem + off_bias);
@@ -412,10 +428,10 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
     constexpr uint16_t CMASK = (uint16_t)((1u << CLUSTER) - 1u);
 
     // ---- one-time setup ----
-    for (int i = threadIdx.x; i < (2 * IMG_BYTES) / 16; i += THREADS)
+    for (int i = threadIdx.x; i < (2 * W::IMG_BYTES) / 16; i += THREADS)
         reinterpret_cast<uint4*>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
-    for (int i = threadIdx.x; i < n_layers * CH; i += THREADS)          // conv layers work in image units (x 2^ACT_SHIFT)
-        s_bias[i] = net.bias[i] * (i < (n_layers - 1) * CH ? ACT_SCALE : 1.0f);
+    for (int i = threadIdx.x; i < n_layers * C; i += THREADS)           // conv layers work in image units (x 2^ACT_SHIFT)
+        s_bias[i] = net.bias[i] * (i < (n_layers - 1) * C ? ACT_SCALE : 1.0f);
     if (threadIdx.x == 0) {
         for (int i = 0; i < nst; ++i) {
             mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, PAIR ? 1 : CLUSTER); mbar_init(bar_pfull + 8 * i, 1);
@@ -429,10 +445,10 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
     cluster_sync_all();                               // peers' barriers exist before anything is multicast
     if (warp == MMA_WARP) {                           // pair mode: a collective of the two CTAs' MMA warps
         if (PAIR) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(TMEM_COLS) : "memory");
+            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(W::TMEM_COLS) : "memory");
             asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
         } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(TMEM_COLS) : "memory");
+            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(W::TMEM_COLS) : "memory");
             asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
         }
     }
@@ -455,29 +471,31 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                 const unsigned char* layer_src = reinterpret_cast<const unsigned char*>(net.wunits) +
                                                  (size_t)(cluster_id % net.replicas) * net.wunits_bytes;
                 for (int layer = 0; layer < n_layers; ++layer) {
-                    const LayerGeom g = layer_geom(layer, n_layers, net.in_ksteps);
+                    const LayerGeom g = layer_geom<C>(layer, n_layers, net.in_ksteps);
                     int dy_bytes = 0;
                     for (int u = 0; u < g.units_per_dy; ++u) dy_bytes += unit_bytes(g, u);
-                    for (int t = 0; t < g.ndy; ++t) {
-                        const int dyi = (t + ROTATE * cluster_id) % g.ndy;
-                        const unsigned char* src = layer_src + (size_t)dyi * dy_bytes;
-                        for (int u = 0; u < g.units_per_dy; ++u) {
-                            const uint32_t bytes = (uint32_t)unit_bytes(g, u);
-                            { long long a = NOW(); mbar_wait(bar_empty + 8 * s, ph ^ 1u, net.error_flag, 1); t_wait += NOW() - a; }
-                            const uint32_t slice = bytes / CLUSTER;
-                            if (PAIR) {                                     // this CTA's half of the rows, kept to itself
-                                mbar_expect_tx(bar_full + 8 * s, slice);
-                                bulk_g2s(s_base + OFF_RING + s * UNIT_SLOT, src + crank * slice, slice, bar_full + 8 * s);
-                            } else {
-                                mbar_expect_tx(bar_full + 8 * s, bytes);   // the whole unit: one slice from every CTA of the cluster
-                                bulk_g2s_multicast(s_base + OFF_RING + s * UNIT_SLOT + crank * slice, src + crank * slice, slice,
-                                                   bar_full + 8 * s, CMASK);
+                    for (int h = 0; h < g.nh; ++h) {                     // output halves (128 channels), one after the other
+                        for (int t = 0; t < g.ndy; ++t) {
+                            const int dyi = (t + ROTATE * cluster_id) % g.ndy;
+                            const unsigned char* src = layer_src + (size_t)dyi * dy_bytes;
+                            for (int u = 0; u < g.units_per_dy; ++u) {
+                                const uint32_t bytes = (uint32_t)unit_bytes(g, u);
+                                { long long a = NOW(); mbar_wait(bar_empty + 8 * s, ph ^ 1u, net.error_flag, 1); t_wait += NOW() - a; }
+                                const uint32_t slice = bytes / CLUSTER;
+                                if (PAIR) {                                     // this CTA's half of the rows, kept to itself
+                                    mbar_expect_tx(bar_full + 8 * s, slice);
+                                    bulk_g2s(s_base + W::OFF_RING + s * UNIT_SLOT, src + crank * slice, slice, bar_full + 8 * s);
+                                } else {
+                                    mbar_expect_tx(bar_full + 8 * s, bytes);   // the whole unit: one slice from every CTA of the cluster
+                                    bulk_g2s_multicast(s_base + W::OFF_RING + s * UNIT_SLOT + crank * slice, src + crank * slice, slice,
+                                                       bar_full + 8 * s, CMASK);
+                                }
+                                src += bytes;
+                                if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
                             }
-                            src += bytes;
-                            if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
                         }
+                        layer_src += (size_t)g.ndy * dy_bytes;
                     }
-                    layer_src += (size_t)g.ndy * dy_bytes;
                 }
             }
             if (net.timing) { net.timing[blockIdx.x * 12 + 8] = t_wait; net.timing[blockIdx.x * 12 + 9] = NOW() - t0; }
@@ -491,7 +509,7 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
         long long t_bar = 0, t_full = 0, t_issue = 0, t_commit = 0, t0 = NOW();
         for (long long tile = blockIdx.x; tile < tile_end; tile += gridDim.x) {
             for (int layer = 0; layer < n_layers; ++layer) {
-                const LayerGeom g = layer_geom(layer, n_layers, net.in_ksteps);
+                const LayerGeom g = layer_geom<C>(layer, n_layers, net.in_ksteps);
                 { long long a = NOW(); named_bar(1, BAR1_THREADS); t_bar += NOW() - a; }   // the layer's input image is complete, the accumulators are drained
                 if (PAIR) {                                                      // ... in the peer CTA as well
                     if (!leader) mbar_arrive_cluster(lead_img);
@@ -503,52 +521,54 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                 const uint32_t idesc = instr_desc_f16(PAIR ? 2 * TILE_M : TILE_M, n1);
                 const bool hi_pass = net.debug < 3 || net.debug == 6, lo_pass = net.debug != 1 && hi_pass;
                 const uint32_t b_lbo = (uint32_t)(2 * nb) * 16u, b_kstep = (2u * b_lbo) >> 4, b_lo_off = ((uint32_t)nb * 16u) >> 4;
-                const uint64_t a_hi0 = smem_desc(s_base + OFF_AHI, CG_STRIDE, 128), a_lo0 = smem_desc(s_base + OFF_ALO, CG_STRIDE, 128);
-                const uint64_t b0 = smem_desc(s_base + OFF_RING, b_lbo, 128);
+                const uint64_t a_hi0 = smem_desc(s_base + W::OFF_AHI, CG_STRIDE, 128), a_lo0 = smem_desc(s_base + W::OFF_ALO, CG_STRIDE, 128);
+                const uint64_t b0 = smem_desc(s_base + W::OFF_RING, b_lbo, 128);
                 constexpr uint32_t A_KSTEP = (2u * CG_STRIDE) >> 4;
-                const uint32_t d_main = tmem;
-                uint32_t acc = 0;                        // 0 for the layer's very first MMA only
-                for (int t = 0; t < g.ndy; ++t) {
-                    const int dyi = (t + ROTATE * cluster_id) % g.ndy;           // same order as the producer
-                    const int dy = g.ndy == 3 ? dyi - 1 : 0;
-                    // in 16-byte slots: two storage rows per board row, or one row of `cols` cells in the linear lattice
-                    const uint32_t a_off = (uint32_t)(16 + (LINEAR ? net.cols : 16) * dy);
-                    for (int u = 0; u < g.units_per_dy; ++u) {
-                        const int nks = unit_ksteps(g, u);
-                        { long long a = NOW(); mbar_wait(bar_full + 8 * s, ph, net.error_flag, 2); t_full += NOW() - a; }
-                        if (PAIR && !leader) {                   // relay: the leader may read this CTA's half now
-                            mbar_arrive_cluster(lead_pfull + 8 * s);
-                            if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
-                            continue;
-                        }
-                        if (PAIR) { long long a = NOW(); mbar_wait_cluster(bar_pfull + 8 * s, ph, net.error_flag, 5); t_full += NOW() - a; }
-                        tc_fence_after();
-                        const long long t_i0 = NOW();
-                        const uint64_t bd = b0 + s * (UNIT_SLOT >> 4);
-                        const uint64_t ah = a_hi0 + a_off + (uint32_t)(UNIT_KS * u) * A_KSTEP, al = a_lo0 + a_off + (uint32_t)(UNIT_KS * u) * A_KSTEP;
-                        if (hi_pass) {
-                            if (nks == UNIT_KS) {
+                for (int h = 0; h < g.nh; ++h) {
+                    const uint32_t d_main = tmem + h * 3 * CH;             // this half's accumulators
+                    uint32_t acc = 0;                        // 0 for the very first MMA of the layer's half only
+                    for (int t = 0; t < g.ndy; ++t) {
+                        const int dyi = (t + ROTATE * cluster_id) % g.ndy;           // same order as the producer
+                        const int dy = g.ndy == 3 ? dyi - 1 : 0;
+                        // in 16-byte slots: two storage rows per board row, or one row of `cols` cells in the linear lattice
+                        const uint32_t a_off = (uint32_t)(16 + (LINEAR ? net.cols : 16) * dy);
+                        for (int u = 0; u < g.units_per_dy; ++u) {
+                            const int nks = unit_ksteps(g, u);
+                            { long long a = NOW(); mbar_wait(bar_full + 8 * s, ph, net.error_flag, 2); t_full += NOW() - a; }
+                            if (PAIR && !leader) {                   // relay: the leader may read this CTA's half now
+                                mbar_arrive_cluster(lead_pfull + 8 * s);
+                                if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
+                                continue;
+                            }
+                            if (PAIR) { long long a = NOW(); mbar_wait_cluster(bar_pfull + 8 * s, ph, net.error_flag, 5); t_full += NOW() - a; }
+                            tc_fence_after();
+                            const long long t_i0 = NOW();
+                            const uint64_t bd = b0 + s * (UNIT_SLOT >> 4);
+                            const uint64_t ah = a_hi0 + a_off + (uint32_t)(UNIT_KS * u) * A_KSTEP, al = a_lo0 + a_off + (uint32_t)(UNIT_KS * u) * A_KSTEP;
+                            if (hi_pass) {
+                                if (nks == UNIT_KS) {
 #pragma unroll
-                                for (int ks = 0; ks < UNIT_KS; ++ks) {
-                                    mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
-                                    mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
-                                    if (lo_pass) mma(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
-                                    acc = 1;
-                                }
-                            } else {
-                                for (int ks = 0; ks < nks; ++ks) {
-                                    mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
-                                    mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
-                                    if (lo_pass) mma(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
-                                    acc = 1;
+                                    for (int ks = 0; ks < UNIT_KS; ++ks) {
+                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
+                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
+                                        if (lo_pass) mma(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
+                                        acc = 1;
+                                    }
+                                } else {
+                                    for (int ks = 0; ks < nks; ++ks) {
+                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
+                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
+                                        if (lo_pass) mma(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
+                                        acc = 1;
+                                    }
                                 }
                             }
+                            const long long t_i1 = NOW();
+                            if (PAIR) umma_commit_pair(bar_empty + 8 * s);      // both producers may refill their halves
+                            else umma_commit_multicast(bar_empty + 8 * s, CMASK);   // every CTA's producer learns that this CTA is done with the unit
+                            t_issue += t_i1 - t_i0; t_commit += NOW() - t_i1;
+                            if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
                         }
-                        const long long t_i1 = NOW();
-                        if (PAIR) umma_commit_pair(bar_empty + 8 * s);      // both producers may refill their halves
-                        else umma_commit_multicast(bar_empty + 8 * s, CMASK);   // every CTA's producer learns that this CTA is done with the unit
-                        t_issue += t_i1 - t_i0; t_commit += NOW() - t_i1;
-                        if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
                     }
                 }
                 if (PAIR) { if (leader) umma_commit_pair(bar_acc); }        // the accumulators of this layer are complete, in both CTAs
@@ -575,8 +595,8 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
         const int cell = r * net.cols + c;
         const bool has_left = c > 0, has_right = c + 1 < net.cols;
         const uint32_t t_lane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-        uint4* a_hi = reinterpret_cast<uint4*>(smem + OFF_AHI);
-        uint4* a_lo = reinterpret_cast<uint4*>(smem + OFF_ALO);
+        uint4* a_hi = reinterpret_cast<uint4*>(smem + W::OFF_AHI);
+        uint4* a_lo = reinterpret_cast<uint4*>(smem + W::OFF_ALO);
         float mx = 0.0f;                                             // largest |image value| this thread produced
         const float vmask = valid ? 1.0f : 0.0f, lmask = has_left ? 1.0f : 0.0f, rmask = has_right ? 1.0f : 0.0f;
         const int cells = net.rows * net.cols, planes = net.in_planes;
@@ -632,17 +652,18 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                 const long long t_layer = NOW();
                 acc_phase ^= 1u;
                 tc_fence_after();
-                const float* bias = s_bias + layer * CH;
+                const float* bias = s_bias + layer * C;
                 if (layer < n_layers - 1 && net.debug >= 5) {
                     // timing experiment: no epilogue work
                 } else if (layer < n_layers - 1) {
                     const bool add_res = layer > 0 && (layer & 1) == 0;      // second conv of a block
                     const bool save_res = (layer & 1) == 0;                  // block input of the next block
 #pragma unroll 1
-                    for (int q = 2 * half; q < 2 * half + 2; ++q) {
+                    for (int q = W::CHUNKS * half; q < W::CHUNKS * half + W::CHUNKS; ++q) {
                         // out[c] = Z_-1[c-1] + Z_0[c] + Z_+1[c+1]; Z_dx = hi half + lo half of accumulator dx
                         float o[16], v[16], w[16];
-                        tmem_ld16x3(t_lane + CH + q * 16, t_lane + q * 16, t_lane + 2 * CH + q * 16, o, v, w);   // dx = 0, -1, +1
+                        const int zc = W::zcol(q);
+                        tmem_ld16x3(t_lane + CH + zc, t_lane + zc, t_lane + 2 * CH + zc, o, v, w);   // dx = 0, -1, +1
                         if (LINEAR) {
                             // publish what the neighbouring warps need: lane 31's Z_-1 (for the next warp's lane 0)
                             // and lane 0's Z_+1 (for the previous warp's lane 31); double-buffered per iteration
@@ -666,14 +687,14 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                         }
                         xbuf ^= 1u;
                         if (add_res) {                                                               // block input (image units), kept in TMEM
-                            tmem_ld16(t_lane + RES_COL + q * 16, v);
+                            tmem_ld16(t_lane + W::RES_COL + q * 16, v);
 #pragma unroll
                             for (int i = 0; i < 16; ++i) o[i] = fmaxf(fmaf(o[i], inv_scale, v[i] + bias[q * 16 + i]), 0.0f) * vmask;
                         } else {
 #pragma unroll
                             for (int i = 0; i < 16; ++i) o[i] = fmaxf(fmaf(o[i], inv_scale, bias[q * 16 + i]), 0.0f) * vmask;
                         }
-                        if (save_res) tmem_st16(t_lane + RES_COL + q * 16, o);
+                        if (save_res) tmem_st16(t_lane + W::RES_COL + q * 16, o);
 #pragma unroll
                         for (int j = 0; j < 2; ++j) {
                             const int cg = q * 2 + j;
@@ -715,38 +736,45 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
     cluster_sync_all();                               // no CTA leaves while peers may still signal its barriers
     if (warp == MMA_WARP) {
         tc_fence_after();
-        if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS) : "memory");
-        else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS) : "memory");
+        if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(W::TMEM_COLS) : "memory");
+        else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(W::TMEM_COLS) : "memory");
     }
 }
 
 #include "evalnet_resident.cuh"
 
 // ---- heads: policy_fc and value_fc1/fc2 over the 1x1-conv activations k_evalnet left in HBM ----
-// 64 boards per CTA, weights staged once in shared memory, 4 boards x 4 outputs per thread.
-constexpr int HB = 64;                        // boards per CTA
+// VH = the value head's hidden width (= the tower width).  HB boards per CTA step, weights staged once in shared memory,
+// BPT boards x 4 outputs per thread: 64 boards with VH = 64, 32 with VH = 128 (its weights and hidden layer take twice
+// the room, and 64 staged boards would not leave Go 9x9 with two policy channels within 227 KB).
+template <int VH> struct Heads {
+    static constexpr int HB = 64 * CH / VH;   // boards per CTA step
+    static constexpr int BPT = HB / 16;       // boards per thread (16 board groups x 16 output groups)
+};
 constexpr int HP_STRIDE = 84;                 // policy weight row stride in floats (up to 82 actions, padded for float4 loads)
 
+template <int VH>
 __global__ void __launch_bounds__(256)
 k_heads(NetDev net, long long batch, const unsigned* __restrict__ d_rows, float* __restrict__ logits, float* __restrict__ value) {
+    constexpr int HB = Heads<VH>::HB, BPT = Heads<VH>::BPT;
     extern __shared__ __align__(16) float hs[];
     if (d_rows) batch = min((long long)*d_rows, batch);
     if ((long long)blockIdx.x * HB >= batch) return;
     const int pc = net.policy_channels, cells = net.rows * net.cols, K = pc * cells, A = net.actions, IN = (pc + 1) * cells;
     float* wp = hs;                           // [K][HP_STRIDE]
-    float* wv = wp + K * HP_STRIDE;           // [cells][64]
-    float* xbuf = wv + cells * 64;            // [2][HB][IN]: the next 64 boards arrive (cp.async) while these are computed
-    float* hid = xbuf + 2 * HB * IN;          // [HB][65]
-    float* wt = hid + HB * 65;                // [K]: weights of output 64 when it is the only one past 64 (the pass action)
+    float* wv = wp + K * HP_STRIDE;           // [cells][VH]
+    float* xbuf = wv + cells * VH;            // [2][HB][IN]: the next HB boards arrive (cp.async) while these are computed
+    float* hid = xbuf + 2 * HB * IN;          // [HB][VH + 1]
+    float* wt = hid + HB * (VH + 1);          // [K]: weights of output 64 when it is the only one past 64 (the pass action)
     const bool lone_tail = A == 65;
     const int a_main = lone_tail ? 64 : A;
     const int t = threadIdx.x;
-    // stages the activations of boards b0 .. b0+63 into buffer `which` (rows past the batch are zero)
+    // stages the activations of boards b0 .. b0+HB-1 into buffer `which` (rows past the batch are zero)
     auto stage = [&](long long b0, int which) {
         if (b0 < batch) {
             const int nb = (int)(batch - b0 < HB ? batch - b0 : HB);
             float* dst = xbuf + which * HB * IN;
-            const float* src = net.head_act + b0 * IN;          // 64 * IN floats per CTA step: 16-byte aligned
+            const float* src = net.head_act + b0 * IN;          // HB * IN floats per CTA step: 16-byte aligned
             const int n16 = nb * IN / 4;
             for (int i = t; i < n16; i += 256)
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(dst + 4 * i)), "l"(src + 4 * i) : "memory");
@@ -756,7 +784,7 @@ k_heads(NetDev net, long long batch, const unsigned* __restrict__ d_rows, float*
     };
     stage((long long)blockIdx.x * HB, 0);
     for (int i = t; i < K * HP_STRIDE; i += 256) { const int k = i / HP_STRIDE, a = i - k * HP_STRIDE; wp[i] = a < A ? net.pfc_wt[k * A + a] : 0.0f; }
-    for (int i = t; i < cells * 64; i += 256) wv[i] = net.vfc1_wt[i];
+    for (int i = t; i < cells * VH; i += 256) wv[i] = net.vfc1_wt[i];
     if (lone_tail) for (int k = t; k < K; k += 256) wt[k] = net.pfc_wt[k * A + 64];
     const int ag = t & 15, bg = t >> 4;       // 16 output groups x 16 board groups
     int cur = 0;
@@ -767,11 +795,11 @@ k_heads(NetDev net, long long batch, const unsigned* __restrict__ d_rows, float*
         asm volatile("cp.async.wait_group 1;" ::: "memory");      // this step's rows have landed
         __syncthreads();
         const float* x = xbuf + cur * HB * IN;
-        // policy_fc: outputs 4*ag .. 4*ag+3 for boards 4*bg .. 4*bg+3 (+ the outputs beyond 64, one per thread row)
+        // policy_fc: outputs 4*ag .. 4*ag+3 for boards BPT*bg .. BPT*bg+BPT-1 (+ the outputs beyond 64, one per thread row)
         for (int a0 = 4 * ag; a0 < a_main; a0 += 64) {
-            float acc[4][4];
+            float acc[BPT][4];
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
+            for (int i = 0; i < BPT; ++i)
 #pragma unroll
                 for (int j = 0; j < 4; ++j) acc[i][j] = 0.0f;
             // four k per step: one 128-bit read of every board's activations (IN and K are multiples of 4 or the tail
@@ -779,14 +807,14 @@ k_heads(NetDev net, long long batch, const unsigned* __restrict__ d_rows, float*
             int k = 0;
             if ((IN & 3) == 0) {
                 for (; k + 4 <= K; k += 4) {
-                    float4 xv[4];
+                    float4 xv[BPT];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) xv[i] = *reinterpret_cast<const float4*>(x + (4 * bg + i) * IN + k);
+                    for (int i = 0; i < BPT; ++i) xv[i] = *reinterpret_cast<const float4*>(x + (BPT * bg + i) * IN + k);
 #pragma unroll
                     for (int kk = 0; kk < 4; ++kk) {
                         const float4 w = *reinterpret_cast<const float4*>(wp + (k + kk) * HP_STRIDE + a0);
 #pragma unroll
-                        for (int i = 0; i < 4; ++i) {
+                        for (int i = 0; i < BPT; ++i) {
                             const float xs = kk == 0 ? xv[i].x : (kk == 1 ? xv[i].y : (kk == 2 ? xv[i].z : xv[i].w));
                             acc[i][0] = fmaf(xs, w.x, acc[i][0]); acc[i][1] = fmaf(xs, w.y, acc[i][1]);
                             acc[i][2] = fmaf(xs, w.z, acc[i][2]); acc[i][3] = fmaf(xs, w.w, acc[i][3]);
@@ -797,21 +825,21 @@ k_heads(NetDev net, long long batch, const unsigned* __restrict__ d_rows, float*
             for (; k < K; ++k) {
                 const float4 w = *reinterpret_cast<const float4*>(wp + k * HP_STRIDE + a0);
 #pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float xv = x[(4 * bg + i) * IN + k];
+                for (int i = 0; i < BPT; ++i) {
+                    const float xv = x[(BPT * bg + i) * IN + k];
                     acc[i][0] = fmaf(xv, w.x, acc[i][0]); acc[i][1] = fmaf(xv, w.y, acc[i][1]);
                     acc[i][2] = fmaf(xv, w.z, acc[i][2]); acc[i][3] = fmaf(xv, w.w, acc[i][3]);
                 }
             }
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
+            for (int i = 0; i < BPT; ++i)
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
-                    if (4 * bg + i < nb && a0 + j < A) logits[(b0 + 4 * bg + i) * A + a0 + j] = acc[i][j] + net.pfc_b[a0 + j];
+                    if (BPT * bg + i < nb && a0 + j < A) logits[(b0 + BPT * bg + i) * A + a0 + j] = acc[i][j] + net.pfc_b[a0 + j];
         }
         if (lone_tail) {
             // Output 64 (Othello's pass) alone would cost the two lanes per warp that own outputs 0..3 a second full pass
-            // over K, i.e. double the policy phase for every warp.  Instead each warp takes 8 boards, the lanes split K
+            // over K, i.e. double the policy phase for every warp.  Instead each warp takes HB / 8 boards, the lanes split K
             // (stride 32, ascending) and a butterfly adds the 32 partial sums: the same order for every board.
             const int wid = t >> 5, ln = t & 31;
             for (int i = 0; i < HB / 8; ++i) {
@@ -823,55 +851,72 @@ k_heads(NetDev net, long long batch, const unsigned* __restrict__ d_rows, float*
                 if (ln == 0 && b < nb) logits[(b0 + b) * A + 64] = sacc + net.pfc_b[64];
             }
         }
-        {   // value_fc1 + ReLU
-            float acc[4][4];
+        {   // value_fc1 + ReLU: outputs 64 * oh + 4*ag .. +3 for boards BPT*bg .. BPT*bg+BPT-1
+            float acc[VH / 64][BPT][4];
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
+            for (int oh = 0; oh < VH / 64; ++oh)
 #pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = 0.0f;
+                for (int i = 0; i < BPT; ++i)
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) acc[oh][i][j] = 0.0f;
             int k = 0;
             if ((IN & 3) == 0 && (K & 3) == 0) {
                 for (; k + 4 <= cells; k += 4) {
-                    float4 xv[4];
+                    float4 xv[BPT];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) xv[i] = *reinterpret_cast<const float4*>(x + (4 * bg + i) * IN + K + k);
+                    for (int i = 0; i < BPT; ++i) xv[i] = *reinterpret_cast<const float4*>(x + (BPT * bg + i) * IN + K + k);
 #pragma unroll
                     for (int kk = 0; kk < 4; ++kk) {
-                        const float4 w = *reinterpret_cast<const float4*>(wv + (k + kk) * 64 + 4 * ag);
 #pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float xs = kk == 0 ? xv[i].x : (kk == 1 ? xv[i].y : (kk == 2 ? xv[i].z : xv[i].w));
-                            acc[i][0] = fmaf(xs, w.x, acc[i][0]); acc[i][1] = fmaf(xs, w.y, acc[i][1]);
-                            acc[i][2] = fmaf(xs, w.z, acc[i][2]); acc[i][3] = fmaf(xs, w.w, acc[i][3]);
+                        for (int oh = 0; oh < VH / 64; ++oh) {
+                            const float4 w = *reinterpret_cast<const float4*>(wv + (k + kk) * VH + 64 * oh + 4 * ag);
+#pragma unroll
+                            for (int i = 0; i < BPT; ++i) {
+                                const float xs = kk == 0 ? xv[i].x : (kk == 1 ? xv[i].y : (kk == 2 ? xv[i].z : xv[i].w));
+                                acc[oh][i][0] = fmaf(xs, w.x, acc[oh][i][0]); acc[oh][i][1] = fmaf(xs, w.y, acc[oh][i][1]);
+                                acc[oh][i][2] = fmaf(xs, w.z, acc[oh][i][2]); acc[oh][i][3] = fmaf(xs, w.w, acc[oh][i][3]);
+                            }
                         }
                     }
                 }
             }
             for (; k < cells; ++k) {
-                const float4 w = *reinterpret_cast<const float4*>(wv + k * 64 + 4 * ag);
 #pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float xv = x[(4 * bg + i) * IN + K + k];
-                    acc[i][0] = fmaf(xv, w.x, acc[i][0]); acc[i][1] = fmaf(xv, w.y, acc[i][1]);
-                    acc[i][2] = fmaf(xv, w.z, acc[i][2]); acc[i][3] = fmaf(xv, w.w, acc[i][3]);
+                for (int oh = 0; oh < VH / 64; ++oh) {
+                    const float4 w = *reinterpret_cast<const float4*>(wv + k * VH + 64 * oh + 4 * ag);
+#pragma unroll
+                    for (int i = 0; i < BPT; ++i) {
+                        const float xv = x[(BPT * bg + i) * IN + K + k];
+                        acc[oh][i][0] = fmaf(xv, w.x, acc[oh][i][0]); acc[oh][i][1] = fmaf(xv, w.y, acc[oh][i][1]);
+                        acc[oh][i][2] = fmaf(xv, w.z, acc[oh][i][2]); acc[oh][i][3] = fmaf(xv, w.w, acc[oh][i][3]);
+                    }
                 }
             }
 #pragma unroll
-            for (int i = 0; i < 4; ++i)
+            for (int oh = 0; oh < VH / 64; ++oh)
 #pragma unroll
-                for (int j = 0; j < 4; ++j) hid[(4 * bg + i) * 65 + 4 * ag + j] = fmaxf(acc[i][j] + net.vfc1_b[4 * ag + j], 0.0f);
+                for (int i = 0; i < BPT; ++i)
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        hid[(BPT * bg + i) * (VH + 1) + 64 * oh + 4 * ag + j] = fmaxf(acc[oh][i][j] + net.vfc1_b[64 * oh + 4 * ag + j], 0.0f);
         }
         __syncthreads();
         if (t < nb) {   // value_fc2 + tanh
-            float s = net.vfc2_w[64];
-            // same summation order for every board (its outputs must not depend on its row); rows of 65 floats: no bank conflicts
-            for (int j = 0; j < 64; ++j) s = fmaf(net.vfc2_w[j], hid[t * 65 + j], s);
+            float s = net.vfc2_w[VH];
+            // same summation order for every board (its outputs must not depend on its row); rows of VH + 1 floats: no bank conflicts
+            for (int j = 0; j < VH; ++j) s = fmaf(net.vfc2_w[j], hid[t * (VH + 1) + j], s);
             value[b0 + t] = tanhf(s);
         }
     }
 }
 
-static inline size_t heads_smem_bytes(int pc, int cells = 64) { return (size_t)(pc * cells * HP_STRIDE + cells * 64 + 2 * HB * (pc + 1) * cells + HB * 65 + pc * cells) * sizeof(float); }
+template <int VH> static inline size_t heads_smem_bytes(int pc, int cells) {
+    constexpr int HB = Heads<VH>::HB;
+    return (size_t)(pc * cells * HP_STRIDE + cells * VH + 2 * HB * (pc + 1) * cells + HB * (VH + 1) + pc * cells) * sizeof(float);
+}
+static inline size_t heads_smem_bytes(int vh, int pc, int cells) {
+    return vh == WIDE_CH ? heads_smem_bytes<WIDE_CH>(pc, cells) : heads_smem_bytes<CH>(pc, cells);
+}
 
 // ---- host: BN folding, hi/lo split, operand packing ------------------------------------------
 // Power-of-two shift that brings the largest |w| of a layer into (2^9, 2^10]: fp16 keeps 11 significant bits
@@ -922,6 +967,19 @@ static void append_resident(std::vector<unsigned short>& out, const std::vector<
                 }
             }
 }
+
+// rows [h * CH, h * CH + CH) of the taps b[t0 .. t0 + n): the weights of output half h of a conv layer (see layer_geom)
+static std::vector<std::vector<float>> output_half(const std::vector<std::vector<float>>& b, int t0, int n, int kk, int h) {
+    std::vector<std::vector<float>> r;
+    for (int t = t0; t < t0 + n; ++t) r.emplace_back(b[t].begin() + (size_t)h * CH * kk, b[t].begin() + (size_t)(h + 1) * CH * kk);
+    return r;
+}
+
+// the streaming kernel's shared memory for a tower of `ch` channels, and the most one CTA of it may take
+static int stream_smem_bytes(int ch, int n_layers, int nst) {
+    return ch == WIDE_CH ? smem_bytes_for<WIDE_CH>(n_layers, nst) : smem_bytes_for<CH>(n_layers, nst);
+}
+static int stream_max_smem(int ch) { return ch == WIDE_CH ? Width<WIDE_CH>::MAX_SMEM : Width<CH>::MAX_SMEM; }
 
 }  // namespace evalnet
 }  // namespace sprl
@@ -980,7 +1038,7 @@ static int check_conv(const sprl_conv_bn_params& c, const char* what) {
 }
 
 static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
-    const int C = CH, P = p->in_planes, L = 2 + 2 * p->blocks;
+    const int C = p->channels, P = p->in_planes, L = 2 + 2 * p->blocks;
     const int in_k = KSTEP_CH * ((3 * P + KSTEP_CH - 1) / KSTEP_CH);      // stem input channels: (dy, plane), see k_evalnet
     const double eps = p->bn_eps > 0 ? p->bn_eps : 1e-5;
     std::vector<unsigned short> units;
@@ -998,10 +1056,10 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
             for (int co = 0; co < C; ++co)
                 for (int ci = 0; ci < cin; ++ci)
                     b[t][(size_t)co * kk + ci] = (float)((double)c.weight[((size_t)co * cin + ci) * 9 + t] * scale[co]);
-        const int shift = weight_shift(b);
+        const int shift = weight_shift(b);            // one shift over all C outputs: both halves share the layer's inv_scale
         inv_scale[layer] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
-        for (int dy = 0; dy < 3; ++dy)
-            append_units(units, std::vector<std::vector<float>>(b.begin() + 3 * dy, b.begin() + 3 * dy + 3), C, kk, shift);
+        for (int h = 0; h < C / CH; ++h)
+            for (int dy = 0; dy < 3; ++dy) append_units(units, output_half(b, 3 * dy, 3, kk, h), CH, kk, shift);
         layers.push_back(LayerW{ std::move(b), C, kk, shift });
     };
     {   // stem: K index dy * P + plane, one unit group with the three dx stacked along N
@@ -1017,7 +1075,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
         }
         const int shift = weight_shift(b);
         inv_scale[0] = std::ldexp(1.0f, -(ACT_SHIFT + shift));
-        append_units(units, b, C, in_k, shift);
+        for (int h = 0; h < C / CH; ++h) append_units(units, output_half(b, 0, 3, in_k, h), CH, in_k, shift);
         layers.push_back(LayerW{ std::move(b), C, in_k, shift });
     }
     for (int i = 0; i < 2 * p->blocks; ++i) conv_layer(p->tower[i], C, C, 1 + i);
@@ -1065,7 +1123,8 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
         for (int b = 0; b < p->blocks; ++b)
             add_group({ RbStage{ RB_CONV, 1 + 2 * b, CH / KSTEP_CH, 0, 0, 0, 0, 0 },
                         RbStage{ RB_CONV, 2 + 2 * b, CH / KSTEP_CH, 0, 1, 0, 0, last_conv == 2 + 2 * b ? 1 : 0 } });
-        bool fits = p->policy_channels <= 2;                      // three head outputs: the fused head sums hold that many
+        // three head outputs: the fused head sums hold that many; 128 channels: one layer's weights alone exceed a CTA pair
+        bool fits = C == CH && p->policy_channels <= 2;
         for (size_t i = 0; i < plan.size(); ++i) fits = fits && plan_smem(plan[i]) <= RB_MAX_SMEM;
         if (fits) {
             std::vector<size_t> w_at;                       // offset (in halfs) of every phase's [rank 0 | rank 1] weights
@@ -1103,13 +1162,13 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
         }
     }
     const int cells = p->rows * p->cols;
-    const int A = p->actions, K = p->policy_channels * cells;
-    std::vector<float> pfc_wt((size_t)K * A), pfc_b(p->policy_fc_b, p->policy_fc_b + A), vfc1_wt((size_t)cells * 64),
-        vfc1_b(p->value_fc1_b, p->value_fc1_b + 64), vfc2_w(p->value_fc2_w, p->value_fc2_w + 64);
+    const int A = p->actions, K = p->policy_channels * cells, VH = p->value_hidden;
+    std::vector<float> pfc_wt((size_t)K * A), pfc_b(p->policy_fc_b, p->policy_fc_b + A), vfc1_wt((size_t)cells * VH),
+        vfc1_b(p->value_fc1_b, p->value_fc1_b + VH), vfc2_w(p->value_fc2_w, p->value_fc2_w + VH);
     for (int a = 0; a < A; ++a)
         for (int k = 0; k < K; ++k) pfc_wt[(size_t)k * A + a] = p->policy_fc_w[(size_t)a * K + k];
-    for (int j = 0; j < 64; ++j)
-        for (int k = 0; k < cells; ++k) vfc1_wt[(size_t)k * 64 + j] = p->value_fc1_w[(size_t)j * cells + k];
+    for (int j = 0; j < VH; ++j)
+        for (int k = 0; k < cells; ++k) vfc1_wt[(size_t)k * VH + j] = p->value_fc1_w[(size_t)j * cells + k];
     vfc2_w.push_back(p->value_fc2_b[0]);
     e->upload_bytes = 0;
     constexpr int REPLICAS = 2;
@@ -1135,7 +1194,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
 #endif
     e->dev.nst = MAX_NST;
     if (getenv("SPRL_EVALNET_NST")) e->dev.nst = std::max(2, std::min(MAX_NST, atoi(getenv("SPRL_EVALNET_NST"))));   // experiments
-    while (e->dev.nst > 2 && smem_bytes_for(L, e->dev.nst) > MAX_SMEM) e->dev.nst -= 1;
+    while (e->dev.nst > 2 && stream_smem_bytes(C, L, e->dev.nst) > stream_max_smem(C)) e->dev.nst -= 1;
     int rc = e->upload(units, &e->dev.wunits);
     if (!rc) rc = e->upload(head_w, &e->dev.head_w);
     if (!rc && !phases.empty()) {
@@ -1170,11 +1229,11 @@ static int validate(const sprl_network_params* p) {
     if (!p) return fail(SPRL_E_INVALID, "null network parameters");
     if (p->rows < 1 || p->cols < 1 || p->cols > 16 || p->rows * p->cols > TILE_M)
         return fail(SPRL_E_INVALID, "the tcgen05 evaluator tiles boards up to 8x8 (two per MMA) or up to %d cells with rows of at most 16 (one per MMA); got %dx%d", TILE_M, p->rows, p->cols);
-    if (p->channels != CH) return fail(SPRL_E_INVALID, "tower width must be %d channels, got %d", CH, p->channels);
+    if (p->channels != CH && p->channels != WIDE_CH) return fail(SPRL_E_INVALID, "tower width must be %d or %d channels, got %d", CH, WIDE_CH, p->channels);
     if (p->blocks < 0 || 2 + 2 * p->blocks > MAX_LAYERS) return fail(SPRL_E_INVALID, "unsupported number of residual blocks %d", p->blocks);
     if (p->in_planes < 1 || 3 * p->in_planes > CH) return fail(SPRL_E_INVALID, "unsupported number of input planes %d (at most %d)", p->in_planes, CH / 3);
-    if (p->policy_channels < 1 || p->policy_channels > 2 || p->value_channels != 1 || p->value_hidden != 64)
-        return fail(SPRL_E_INVALID, "unsupported head shape (policy channels %d, value channels %d, value hidden %d)",
+    if (p->policy_channels < 1 || p->policy_channels > 2 || p->value_channels != 1 || p->value_hidden != p->channels)
+        return fail(SPRL_E_INVALID, "unsupported head shape (policy channels %d, value channels %d, value hidden %d; the value hidden layer must be as wide as the tower)",
                     p->policy_channels, p->value_channels, p->value_hidden);
     if (p->actions < 1 || p->actions > HP_STRIDE) return fail(SPRL_E_INVALID, "unsupported action count %d", p->actions);
     int rc = check_conv(p->stem, "stem");
@@ -1209,13 +1268,16 @@ int sprl_evalnet_create(int device, const sprl_network_params* params, sprl_eval
     e->sm_count = prop.multiProcessorCount;
     if (getenv("SPRL_EVALNET_MAX_CTAS")) e->max_ctas = atoi(getenv("SPRL_EVALNET_MAX_CTAS"));
     if (getenv("SPRL_EVALNET_PATH")) e->path = atoi(getenv("SPRL_EVALNET_PATH"));      // experiments: 1 streaming, 2 resident
-    err = cudaFuncSetAttribute(k_evalnet<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM);
-    if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAX_SMEM);
+    err = cudaFuncSetAttribute(k_evalnet<false, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<CH>::MAX_SMEM);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet<true, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<CH>::MAX_SMEM);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet<false, WIDE_CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<WIDE_CH>::MAX_SMEM);
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet<true, WIDE_CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<WIDE_CH>::MAX_SMEM);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet_resident<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, RB_MAX_SMEM);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet_resident<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, RB_MAX_SMEM);
     if (err != cudaSuccess) { delete e; return fail(SPRL_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(err)); }
-    if (heads_smem_bytes(params->policy_channels, params->rows * params->cols) > 227 * 1024) { delete e; return fail(SPRL_E_INVALID, "head layers of %d channels x %d cells do not fit k_heads' shared memory", params->policy_channels, params->rows * params->cols); }
-    err = cudaFuncSetAttribute(k_heads, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);   // the attribute is per process: always the maximum, whatever this evaluator's board
+    if (heads_smem_bytes(params->value_hidden, params->policy_channels, params->rows * params->cols) > 227 * 1024) { delete e; return fail(SPRL_E_INVALID, "head layers of %d channels x %d cells do not fit k_heads' shared memory", params->policy_channels, params->rows * params->cols); }
+    err = cudaFuncSetAttribute(k_heads<CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);   // the attribute is per process: always the maximum, whatever this evaluator's board
+    if (err == cudaSuccess) err = cudaFuncSetAttribute(k_heads<WIDE_CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (err != cudaSuccess) { delete e; return fail(SPRL_E_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(err)); }
     rc = pack_and_upload(e, params);
     if (rc) { e->release(); delete e; return rc; }
@@ -1229,7 +1291,7 @@ int sprl_evalnet_update(sprl_evalnet* e, const sprl_network_params* params) {
     int rc = validate(params);
     if (rc) return rc;
     if (params->rows != e->rows || params->cols != e->cols || params->in_planes != e->in_planes || params->blocks != e->blocks || params->actions != e->actions ||
-        params->policy_channels != e->policy_channels)
+        params->policy_channels != e->policy_channels || params->channels != e->channels)
         return fail(SPRL_E_INVALID, "sprl_evalnet_update: the network shape changed");
     rc = use_device(e->device);
     if (rc) return rc;
@@ -1301,26 +1363,33 @@ int sprl_evalnet_forward_counted(sprl_evalnet* e, const float* d_in, const uint3
             if (err != cudaSuccess) break;
         }
     } else {
-    const int max_grid = e->sm_count * CTAS_PER_SM / CLUSTER * CLUSTER;
+    const bool wide = e->channels == WIDE_CH;
+    const int max_grid = e->sm_count * (wide ? Width<WIDE_CH>::CTAS_PER_SM : Width<CH>::CTAS_PER_SM) / CLUSTER * CLUSTER;
     const int grid = (int)std::min<long long>((tiles + CLUSTER - 1) / CLUSTER * CLUSTER, max_grid);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(THREADS);
-    cfg.dynamicSmemBytes = (size_t)smem_bytes_for(e->dev.n_layers, e->dev.nst);
+    cfg.dynamicSmemBytes = (size_t)stream_smem_bytes(e->channels, e->dev.n_layers, e->dev.nst);
     cfg.stream = (cudaStream_t)cuda_stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = CLUSTER; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    err = e->dev.linear ? cudaLaunchKernelEx(&cfg, k_evalnet<true>, e->dev, d_in, (long long)batch, (const unsigned*)d_rows, d_logits, d_value)
-                        : cudaLaunchKernelEx(&cfg, k_evalnet<false>, e->dev, d_in, (long long)batch, (const unsigned*)d_rows, d_logits, d_value);
+    auto* kernel = wide ? (e->dev.linear ? k_evalnet<true, WIDE_CH> : k_evalnet<false, WIDE_CH>)
+                        : (e->dev.linear ? k_evalnet<true, CH> : k_evalnet<false, CH>);
+    err = cudaLaunchKernelEx(&cfg, kernel, e->dev, d_in, (long long)batch, (const unsigned*)d_rows, d_logits, d_value);
     e->launches += 1;
     if (err == cudaSuccess) err = cudaGetLastError();
     }
     if (err == cudaSuccess) {
-        const int hgrid = (int)std::min<long long>((batch + HB - 1) / HB, (long long)e->sm_count);     // one resident CTA per SM (its weights are staged once)
-        k_heads<<<hgrid, 256, heads_smem_bytes(e->policy_channels, e->rows * e->cols), (cudaStream_t)cuda_stream>>>(e->dev, (long long)batch, (const unsigned*)d_rows, d_logits, d_value);
+        const int hb = e->value_hidden == WIDE_CH ? Heads<WIDE_CH>::HB : Heads<CH>::HB;
+        const int hgrid = (int)std::min<long long>((batch + hb - 1) / hb, (long long)e->sm_count);     // one resident CTA per SM (its weights are staged once)
+        const size_t hsmem = heads_smem_bytes(e->value_hidden, e->policy_channels, e->rows * e->cols);
+        if (e->value_hidden == WIDE_CH)
+            k_heads<WIDE_CH><<<hgrid, 256, hsmem, (cudaStream_t)cuda_stream>>>(e->dev, (long long)batch, (const unsigned*)d_rows, d_logits, d_value);
+        else
+            k_heads<CH><<<hgrid, 256, hsmem, (cudaStream_t)cuda_stream>>>(e->dev, (long long)batch, (const unsigned*)d_rows, d_logits, d_value);
         e->launches += 1;
         err = cudaGetLastError();
     }
@@ -1373,7 +1442,7 @@ int sprl_evalnet_info(sprl_evalnet* e, int64_t* upload_bytes, int32_t* ring_stag
     if (upload_bytes) *upload_bytes = e->upload_bytes;
     if (ring_stages) *ring_stages = e->dev.nst;
     if (smem_bytes) {
-        *smem_bytes = smem_bytes_for(e->dev.n_layers, e->dev.nst);
+        *smem_bytes = stream_smem_bytes(e->channels, e->dev.n_layers, e->dev.nst);
         if (!e->phases.empty() && e->path != SPRL_EVALNET_PATH_STREAMING) {      // the resident kernel: its largest phase
             *smem_bytes = 0;
             for (const RbPhase& ph : e->phases) *smem_bytes = std::max(*smem_bytes, rb_smem_bytes(ph, e->dev.linear != 0));
