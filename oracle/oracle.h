@@ -137,6 +137,29 @@ typedef struct {
 
 int oracle_match(const oracle_selfplay_cfg agents[2], uint64_t first_game, int ngames, oracle_match_out* out);
 
+/* Shape of the searches (counters only: they change no other output).  A descent's depth is the number of edges
+ * chosen below the decision node.  The search kernel records up to 32 edges of a descent for its parallel backup and
+ * backs deeper ones up by parent links; its leaf-batch deduplication compares the first 32 queue entries only.
+ * A separate struct, filled by the _ex entry points, so that callers of the structs above keep their layout. */
+#define ODEPTH_BINS 128
+typedef struct {
+    int64_t total_traversals, total_evals;
+    int64_t leaves_terminal, leaves_gray, leaves_empty;
+    double select_depth_sum, select_legal_sum;
+    int32_t select_depth_max;
+    int64_t depth_hist[ODEPTH_BINS];    /* descents by depth, the last bin counts every depth >= 127 */
+    int64_t deep_terminal, deep_gray, deep_queued;   /* descents of >= 32 edges by how their leaf was handled */
+    int32_t queue_max;                  /* most leaves queued by one searchAndGetLeaves call */
+    int64_t dup_total;                  /* queued leaves already queued earlier in the same batch */
+    int64_t dup_first32;                /* the same, counted only among the first 32 entries of each batch */
+} oracle_search_stats;
+
+/* oracle_selfplay / oracle_match that also fill `search` (may be NULL); in a match it sums both agents' searches. */
+int oracle_selfplay_ex(const oracle_selfplay_cfg* cfg, uint64_t first_game, int ngames, oracle_selfplay_out* out,
+                       oracle_search_stats* search);
+int oracle_match_ex(const oracle_selfplay_cfg agents[2], uint64_t first_game, int ngames, oracle_match_out* out,
+                    oracle_search_stats* search);
+
 /* .npy v1.0 writer restated from utils/npy.hpp:430-476,616-639 (float32, C order). */
 int oracle_write_npy_f32(const char* path, const float* data, const uint64_t* shape, int ndim);
 

@@ -182,6 +182,8 @@ typedef struct {
     onode* decision;        /* m_decisionNode */
     float root_P[1], root_W[1], root_N[1];   /* tree-level dummy edge, uct/UCTTree.hpp:301 (action 0) */
     oracle_selfplay_out* stats;
+    oracle_search_stats* search;    /* may be NULL */
+    int last_depth;         /* edges of the last descent (search stats only) */
 } otree;
 
 static void node_attach_stats(onode* n) {
@@ -259,11 +261,14 @@ static onode* tree_select_leaf(otree* t) {
     int depth = 0;
     while (cur->expanded && !cur->terminal) {
         int a = uct_best_action(t, cur);
-        if (t->stats) {
+        if (t->stats || t->search) {
             int nl = 0;
             for (int i = 0; i < t->gi->actions; ++i) nl += cur->mask[i] != 0.0f;
-            t->stats->select_legal_sum += nl;
-            t->stats->select_nodes += 1;
+            if (t->stats) {
+                t->stats->select_legal_sum += nl;
+                t->stats->select_nodes += 1;
+            }
+            if (t->search) t->search->select_legal_sum += nl;
         }
         *cur->own_N += 1;
         *cur->own_W -= 1;
@@ -273,6 +278,7 @@ static onode* tree_select_leaf(otree* t) {
     *cur->own_N += 1;
     *cur->own_W -= 1;
     if (t->stats) t->stats->select_depth_sum += depth;
+    t->last_depth = depth;
     return cur;
 }
 
@@ -284,6 +290,34 @@ static void tree_backup(otree* t, onode* node, float valueEstimate) {
     while (cur != stop) {
         *cur->own_W += 1 + estimate * ((cur->player == O_ZERO) ? 1 : -1);
         cur = cur->parent;
+    }
+}
+
+/* search stats: the last descent ended at a leaf handled as `kind` (0 terminal, 1 gray, 2 queued as entry `k` of
+ * `leaves`) */
+static void note_descent(otree* t, int kind, onode** leaves, int k) {
+    oracle_search_stats* s = t->search;
+    if (!s) return;
+    int d = t->last_depth;
+    s->select_depth_sum += d;
+    if (d > s->select_depth_max) s->select_depth_max = d;
+    s->depth_hist[d < ODEPTH_BINS - 1 ? d : ODEPTH_BINS - 1] += 1;
+    if (kind == 0) s->leaves_terminal += 1;
+    else if (kind == 1) s->leaves_gray += 1;
+    else s->leaves_empty += 1;
+    if (d >= 32) {
+        if (kind == 0) s->deep_terminal += 1;
+        else if (kind == 1) s->deep_gray += 1;
+        else s->deep_queued += 1;
+    }
+    if (kind == 2) {
+        if (k + 1 > s->queue_max) s->queue_max = k + 1;
+        for (int j = 0; j < k; ++j) {
+            if (leaves[j] != leaves[k]) continue;
+            s->dup_total += 1;
+            if (k < 32) s->dup_first32 += 1;
+            break;
+        }
     }
 }
 
@@ -299,15 +333,18 @@ static int tree_search(otree* t, onode** leaves, int* nleaves) {
             og_rewards(leaf, rewards);
             tree_backup(t, leaf, rewards[leaf->player]);
             if (t->stats) t->stats->leaves_terminal++;
+            note_descent(t, 0, leaves, 0);
             continue;
         } else if (leaf->evaluated) {
             uct_expand(t, leaf, t->cfg->add_noise && leaf == t->decision);
             tree_backup(t, leaf, leaf->net_value);
             if (t->stats) t->stats->leaves_gray++;
+            note_descent(t, 1, leaves, 0);
             continue;
         } else {
             leaves[(*nleaves)++] = leaf;
             if (t->stats) t->stats->leaves_empty++;
+            note_descent(t, 2, leaves, *nleaves - 1);
         }
         if (*nleaves >= t->cfg->max_queue) break;
     }
@@ -341,6 +378,7 @@ static void tree_evaluate_and_backprop(otree* t, onode** leaves, int n) {
     }
     evaluate_batch(t->cfg, gi, states, (const float (*)[OG_MAXA])masks, n, policy, value);
     if (t->stats) t->stats->total_evals += n;
+    if (t->search) t->search->total_evals += n;
     for (int i = 0; i < n; ++i) {
         onode* leaf = leaves[i];
         float pol[OG_MAXA];
@@ -378,14 +416,15 @@ static void tree_advance(otree* t, int action) {
 #define PUT(arr, idx, val) do { if (arr) (arr)[idx] = (val); } while (0)
 
 /* selfplay/SelfPlay.hpp:50-192 for one game; appends to `out` */
-static int self_play_game(const oracle_selfplay_cfg* cfg, uint64_t game_id, int gslot, oracle_selfplay_out* out) {
+static int self_play_game(const oracle_selfplay_cfg* cfg, uint64_t game_id, int gslot, oracle_selfplay_out* out,
+                          oracle_search_stats* search) {
     const ogame_info* gi = og_info(cfg->game);
     int A = gi->actions, B = gi->cells, S = cfg->use_sym ? gi->nsym : 1;
     int plane = (2 * gi->history + 1) * B;
     orng_t rng = { cfg->seed, game_id, 0 };
     otree t;
     memset(&t, 0, sizeof(t));
-    t.cfg = cfg; t.gi = gi; t.game = cfg->game; t.rng = &rng; t.stats = out;
+    t.cfg = cfg; t.gi = gi; t.game = cfg->game; t.rng = &rng; t.stats = out; t.search = search;
     t.game_root = og_new_root(cfg->game);
     t.game_root->own_N = &t.root_N[0];
     t.game_root->own_W = &t.root_W[0];
@@ -419,6 +458,7 @@ static int self_play_game(const oracle_selfplay_cfg* cfg, uint64_t game_id, int 
             traversals += trav;
         }
         out->total_traversals += traversals;
+        if (search) search->total_traversals += traversals;
 
         int64_t m = out->n_moves;
         for (int a = 0; a < A; ++a) {
@@ -479,7 +519,8 @@ static int self_play_game(const oracle_selfplay_cfg* cfg, uint64_t game_id, int 
     return rc;
 }
 
-int oracle_selfplay(const oracle_selfplay_cfg* cfg, uint64_t first_game, int ngames, oracle_selfplay_out* out) {
+int oracle_selfplay_ex(const oracle_selfplay_cfg* cfg, uint64_t first_game, int ngames, oracle_selfplay_out* out,
+                       oracle_search_stats* search) {
     if (!og_info(cfg->game)) return -2;
     if (cfg->evaluator == OE_CALLBACK && !cfg->eval_cb) return -2;
     out->n_moves = out->n_samples = 0;
@@ -487,24 +528,30 @@ int oracle_selfplay(const oracle_selfplay_cfg* cfg, uint64_t first_game, int nga
     out->select_depth_sum = out->select_legal_sum = 0.0;
     out->select_nodes = 0;
     out->leaves_terminal = out->leaves_gray = out->leaves_empty = 0;
+    if (search) memset(search, 0, sizeof(*search));
     for (int g = 0; g < ngames; ++g) {          /* selfplay/SelfPlay.hpp:203-248: games in order, concatenated */
-        int rc = self_play_game(cfg, first_game + (uint64_t)g, g, out);
+        int rc = self_play_game(cfg, first_game + (uint64_t)g, g, out, search);
         if (rc) return rc;
     }
     return 0;
 }
 
+int oracle_selfplay(const oracle_selfplay_cfg* cfg, uint64_t first_game, int ngames, oracle_selfplay_out* out) {
+    return oracle_selfplay_ex(cfg, first_game, ngames, out, NULL);
+}
+
 /* ------------------------------------------------------------------ match play */
-static void match_tree_init(otree* t, const oracle_selfplay_cfg* cfg, orng_t* rng) {
+static void match_tree_init(otree* t, const oracle_selfplay_cfg* cfg, orng_t* rng, oracle_search_stats* search) {
     memset(t, 0, sizeof(*t));
-    t->cfg = cfg; t->gi = og_info(cfg->game); t->game = cfg->game; t->rng = rng; t->stats = NULL;
+    t->cfg = cfg; t->gi = og_info(cfg->game); t->game = cfg->game; t->rng = rng; t->stats = NULL; t->search = search;
     t->game_root = og_new_root(cfg->game);
     t->game_root->own_N = &t->root_N[0];
     t->game_root->own_W = &t->root_W[0];
     t->decision = t->game_root;
 }
 
-int oracle_match(const oracle_selfplay_cfg agents[2], uint64_t first_game, int ngames, oracle_match_out* out) {
+int oracle_match_ex(const oracle_selfplay_cfg agents[2], uint64_t first_game, int ngames, oracle_match_out* out,
+                    oracle_search_stats* search) {
     const ogame_info* gi = og_info(agents[0].game);
     if (!gi) return -2;
     int A = gi->actions;
@@ -516,14 +563,15 @@ int oracle_match(const oracle_selfplay_cfg agents[2], uint64_t first_game, int n
         cfg[k].dir_eps = 0.25f; cfg[k].dir_alpha = 0.1f; cfg[k].add_noise = 1; cfg[k].u_weight = 1.0f;
     }
     out->n_moves = 0; out->wins[0] = out->wins[1] = 0; out->draws = 0;
+    if (search) memset(search, 0, sizeof(*search));
     onode** leaves = (onode**)malloc(sizeof(onode*) * (size_t)(cfg[0].max_batch > 0 ? cfg[0].max_batch : 1));
     int rc = 0;
     for (int g = 0; g < ngames && rc == 0; ++g) {
         uint64_t tg = first_game + (uint64_t)g;
         orng_t rng = { cfg[0].seed, tg, 0 };
         otree tree[2];
-        match_tree_init(&tree[0], &cfg[0], &rng);
-        match_tree_init(&tree[1], &cfg[1], &rng);
+        match_tree_init(&tree[0], &cfg[0], &rng, search);
+        match_tree_init(&tree[1], &cfg[1], &rng, search);
         int moves = 0;
         while (!tree[0].decision->terminal) {   /* evaluate/play.hpp:38-57 */
             if (out->n_moves >= out->cap_moves) { rc = -1; break; }
@@ -538,6 +586,7 @@ int oracle_match(const oracle_selfplay_cfg agents[2], uint64_t first_game, int n
                 if (nleaves > 0) tree_evaluate_and_backprop(t, leaves, nleaves);
                 traversals += trav;
             }
+            if (search) search->total_traversals += traversals;
             int64_t m = out->n_moves;
             int action = 0;                     /* std::max_element: first of the largest, :92-93 */
             for (int a = 0; a < A; ++a) {
@@ -570,6 +619,10 @@ int oracle_match(const oracle_selfplay_cfg agents[2], uint64_t first_game, int n
     }
     free(leaves);
     return rc;
+}
+
+int oracle_match(const oracle_selfplay_cfg agents[2], uint64_t first_game, int ngames, oracle_match_out* out) {
+    return oracle_match_ex(agents, first_game, ngames, out, NULL);
 }
 
 /* ------------------------------------------------------------------ npy I/O */

@@ -65,6 +65,23 @@ class SelfplayCfg(C.Structure):
                 ("caller_moves", C.c_int)]
 
 
+DEPTH_BINS = 128
+
+
+class SearchStats(C.Structure):
+    """oracle_search_stats: totals and shape of the searches (descent depths, deep descents by ending, duplicates)."""
+    _fields_ = [("total_traversals", C.c_int64), ("total_evals", C.c_int64), ("leaves_terminal", C.c_int64),
+                ("leaves_gray", C.c_int64), ("leaves_empty", C.c_int64), ("select_depth_sum", C.c_double),
+                ("select_legal_sum", C.c_double), ("select_depth_max", C.c_int32), ("depth_hist", C.c_int64 * DEPTH_BINS),
+                ("deep_terminal", C.c_int64), ("deep_gray", C.c_int64), ("deep_queued", C.c_int64),
+                ("queue_max", C.c_int32), ("dup_total", C.c_int64), ("dup_first32", C.c_int64)]
+
+    def as_dict(self):
+        d = {n: getattr(self, n) for n, _ in self._fields_}
+        d["depth_hist"] = np.array(self.depth_hist[:], np.int64)
+        return d
+
+
 class MatchOut(C.Structure):
     _fields_ = [("cap_moves", C.c_int64), ("game_moves", C.c_void_p), ("game_winner", C.c_void_p),
                 ("game_rng_draws", C.c_void_p), ("move_N", C.c_void_p), ("move_W", C.c_void_p), ("move_P", C.c_void_p),
@@ -152,8 +169,9 @@ def replay(game, actions):
 
 def selfplay(game, evaluator, seed, first_game, ngames, sims, max_batch, max_queue, eps=0.25, alpha=0.3,
              add_noise=True, use_sym=True, init_q=OQ_PARENT, u_weight=1.1, eval_fn=None, max_moves_per_game=200,
-             fix_symmetry_mask=False, caller_moves=False):
-    """Run the oracle's selfPlay for `ngames` games; returns a dict shaped like a ref_trace selfplay trace."""
+             fix_symmetry_mask=False, caller_moves=False, search_stats=False):
+    """Run the oracle's selfPlay for `ngames` games; returns a dict shaped like a ref_trace selfplay trace, plus
+    "stats": the totals of oracle_selfplay_out and, with search_stats, the fields of oracle_search_stats."""
     gi = game_info(game)
     S = gi.nsym if use_sym else 1
     cap_m = ngames * max_moves_per_game
@@ -186,7 +204,11 @@ def selfplay(game, evaluator, seed, first_game, ngames, sims, max_batch, max_que
     out = SelfplayOut(cap_moves=cap_m, cap_samples=cap_s)
     for k, v in arr.items():
         setattr(out, k, v.ctypes.data)
-    rc = lib().oracle_selfplay(C.byref(cfg), C.c_uint64(first_game), C.c_int(ngames), C.byref(out))
+    search = SearchStats()
+    if search_stats:
+        rc = lib().oracle_selfplay_ex(C.byref(cfg), C.c_uint64(first_game), C.c_int(ngames), C.byref(out), C.byref(search))
+    else:
+        rc = lib().oracle_selfplay(C.byref(cfg), C.c_uint64(first_game), C.c_int(ngames), C.byref(out))
     assert rc == 0, rc
     M, N = out.n_moves, out.n_samples
     res = {}
@@ -201,6 +223,8 @@ def selfplay(game, evaluator, seed, first_game, ngames, sims, max_batch, max_que
                         select_depth_sum=out.select_depth_sum, select_legal_sum=out.select_legal_sum,
                         select_nodes=out.select_nodes, leaves_terminal=out.leaves_terminal,
                         leaves_gray=out.leaves_gray, leaves_empty=out.leaves_empty)
+    if search_stats:
+        res["stats"] = dict(search.as_dict(), **res["stats"])
     return res
 
 
@@ -215,9 +239,10 @@ def _make_eval_cb(gi, eval_fn):
     return EVAL_CB(_cb)
 
 
-def match(game, agents, seed, first_game, ngames, sims, max_batch, max_queue, max_moves_per_game=200):
+def match(game, agents, seed, first_game, ngames, sims, max_batch, max_queue, max_moves_per_game=200, search_stats=False):
     """Run the oracle's match play.  agents = two dicts with keys evaluator, use_sym, init_q and optionally
-    hash_salt / eval_fn.  Returns a dict shaped like a ref_trace match trace (+ wins, draws)."""
+    hash_salt / eval_fn.  Returns a dict shaped like a ref_trace match trace (+ wins, draws, and with search_stats
+    "stats": the fields of oracle_search_stats over both agents' searches)."""
     gi = game_info(game)
     A = gi.actions
     cap_m = ngames * max_moves_per_game
@@ -240,11 +265,17 @@ def match(game, agents, seed, first_game, ngames, sims, max_batch, max_queue, ma
     out = MatchOut(cap_moves=cap_m)
     for k, v in arr.items():
         setattr(out, k, v.ctypes.data)
-    rc = lib().oracle_match(cfgs, C.c_uint64(first_game), C.c_int(ngames), C.byref(out))
+    search = SearchStats()
+    if search_stats:
+        rc = lib().oracle_match_ex(cfgs, C.c_uint64(first_game), C.c_int(ngames), C.byref(out), C.byref(search))
+    else:
+        rc = lib().oracle_match(cfgs, C.c_uint64(first_game), C.c_int(ngames), C.byref(out))
     assert rc == 0, rc
     res = {k: (v[:out.n_moves] if k.startswith("move_") else v) for k, v in arr.items()}
     res["wins"] = (out.wins[0], out.wins[1])
     res["draws"] = out.draws
+    if search_stats:
+        res["stats"] = search.as_dict()
     return res
 
 

@@ -276,7 +276,8 @@ def test_external_evaluator_bit_exact(game, sims, b, q, alpha, ngames, graph):
     compare_selfplay(ref, got)
     assert st["sims"] == ref["stats"]["total_traversals"] and st["evals"] == ref["stats"]["total_evals"]
     # quirk Q4: the fresh root alone is queued max_queue times in the first batch of a game; the copies are counted like the
-    # reference's getNumEvals but share one evaluator row
+    # reference's getNumEvals but share one evaluator row.  The bound holds for q <= 32: only the first 32 entries of a
+    # batch are compared (tests/test_search_edges.py checks the exact count for wider queues)
     assert (q - 1) * ngames <= st["leaves_duplicate"] < st["evals"] // 2
 
 
