@@ -87,7 +87,7 @@ def load():
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("SPRL_B200_LIB") or _build.LIB_PATH      # SPRL_B200_LIB: a build variant (timing experiments)
+    path = os.environ.get("SPRL_B200_LIB") or _build.LIB_PATH      # SPRL_B200_LIB: another build of the library, e.g. a parent commit's for A/B runs
     if path == _build.LIB_PATH and (not os.path.exists(path) or os.environ.get("SPRL_B200_REBUILD")):
         _build.build_library()
     lib = C.CDLL(path)

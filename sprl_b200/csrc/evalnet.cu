@@ -77,10 +77,7 @@ constexpr int ACT_SHIFT = 4;                 // activations are stored x 2^ACT_S
 constexpr float ACT_SCALE = 16.0f, HALF_MAX = 65504.0f;
 constexpr int SLOTS = 160;                   // 20 storage rows x 8 cells
 constexpr int CG_STRIDE = SLOTS * 16;        // bytes per channel group of the image
-#ifndef SPRL_EVALNET_UNIT_KSTEPS
-#define SPRL_EVALNET_UNIT_KSTEPS 2
-#endif
-constexpr int UNIT_KS = SPRL_EVALNET_UNIT_KSTEPS;      // k-steps (16 input channels each) per weight unit
+constexpr int UNIT_KS = 2;                   // k-steps (16 input channels each) per weight unit
 constexpr int UNIT_BYTES = UNIT_KS * 2 * (6 * CH) * 16; // [K chunk of 8][3 dx x (hi, lo) x 64 rows][8 halfs]: 24 KB = 32 input channels of one dy
 constexpr int MAX_NST = 12;                  // ring stages (as many as shared memory holds)
 constexpr int MAX_LAYERS = 16;
@@ -92,33 +89,8 @@ constexpr int EPI_WARPS = 8;                 // two warps per TMEM lane quarter,
 constexpr int MMA_WARP = EPI_WARPS, PRODUCER_WARP = EPI_WARPS + 1;
 constexpr int THREADS = (EPI_WARPS + 2) * 32;
 constexpr int BAR1_THREADS = (EPI_WARPS + 1) * 32;   // epilogue warps + MMA warp
-#ifndef SPRL_EVALNET_CLUSTER
-#define SPRL_EVALNET_CLUSTER 2
-#endif
-constexpr int CLUSTER = SPRL_EVALNET_CLUSTER;  // CTAs sharing one multicast weight stream
-#ifndef SPRL_EVALNET_ROTATE
-#define SPRL_EVALNET_ROTATE 0
-#endif
-// 1: clusters walk the vertical taps of a layer in different rotations (spreads the L2 reads of the weight stream, but
-// the fp32 accumulation order of a board then depends on which CTA evaluates it).  0: one order everywhere, so a
-// board's outputs do not depend on its row in the batch -- self-play with compact leaf rows stays reproducible.
-constexpr int ROTATE = SPRL_EVALNET_ROTATE;
-#ifndef SPRL_EVALNET_PAIR
-#define SPRL_EVALNET_PAIR 0
-#endif
-// Experiment switch, off by default.  CTA pair (tcgen05 cta_group::2): the two CTAs of a cluster run ONE MMA of
-// M = 256 -- each supplies its own tile (128 rows of A, its own accumulators) and HALF of the weight rows (B), so a
-// CTA stores and reads only half of every weight unit.  The leader (cluster rank 0) issues; the peer's MMA warp relays
-// "my half has landed" / "my image is ready" to the leader's barriers.  Correct (1.4e-7) and the MMAs issue 28 %
-// faster, but the two tiles of a pair then move in lockstep and the relay adds latency: 1.65 ms against 1.45 ms for
-// two independent CTAs (profiles/r1h_evalnet_pair_variants.txt), so the independent CTAs stay the default.
-constexpr bool PAIR = SPRL_EVALNET_PAIR != 0;
-static_assert(!PAIR || CLUSTER == 2, "the CTA pair is a cluster of two");
-constexpr int UNIT_SLOT = PAIR ? UNIT_BYTES / 2 : UNIT_BYTES;   // bytes of a ring stage in one CTA
+constexpr int CLUSTER = 2;                   // CTAs sharing one multicast weight stream
 constexpr int RES_COL = 3 * CH;              // resident kernel: the block input of the current residual block, fp32, one cell per lane
-#ifndef SPRL_EVALNET_CTAS_PER_SM
-#define SPRL_EVALNET_CTAS_PER_SM 2
-#endif
 
 // Streaming kernel (k_evalnet) geometry of a tower of C channels.  The C outputs of a conv layer are C / 64 output
 // halves of 64 channels; every half is the same N = 192 MMA (3 dx x 64) into its own 192 TMEM columns
@@ -129,10 +101,11 @@ template <int C> struct Width {
     static constexpr int IMG_BYTES = (C / KCH) * CG_STRIDE;  // 20,480 / 40,960
     static constexpr int TMEM_COLS = NH == 1 ? 256 : 512;
     static constexpr int RES_COL = 3 * CH * NH;              // the block input of the current residual block, fp32, one cell per lane
-    static constexpr int CTAS_PER_SM = NH == 1 ? SPRL_EVALNET_CTAS_PER_SM : 1;   // resident CTAs per SM
+    static constexpr int CTAS_PER_SM = NH == 1 ? 2 : 1;      // resident CTAs per SM
     static constexpr int MAX_SMEM = (232448 - (CTAS_PER_SM - 1) * 1024) / CTAS_PER_SM;   // 227 KB per SM, 1 KB reserved per extra CTA
     static constexpr int CHUNKS = C / 32;                    // 16-channel epilogue chunks per warp (two warps per lane quarter)
-    // shared memory map (bytes); the ring, the biases and the barriers follow at run-time offsets
+    // shared memory map (bytes); the ring, the biases, the TMEM address (16 B), the linear lattice's neighbour scratch
+    // and the barriers (full[nst], empty[nst], acc) follow at run-time offsets
     static constexpr int OFF_AHI = 0, OFF_ALO = IMG_BYTES, OFF_RING = 2 * IMG_BYTES;
     // TMEM column of accumulator dx = -1 for channels [16 q, 16 q + 16); dx = 0 and +1 follow at +64 and +128
     __device__ static constexpr int zcol(int q) { return q * 16 + (NH > 1 ? (q >> 2) * 2 * CH : 0); }
@@ -162,14 +135,11 @@ struct NetDev {
     unsigned long long* error_flag;   // [0] pipeline barrier time-out, [1] an activation left the fp16-split range
     const float* inv_scale;  // [MAX_LAYERS] 2^-(ACT_SHIFT + weight shift of the layer): accumulator -> real units.  In device
                              // memory, not in this by-value struct: a captured CUDA graph must see the scales of update()
-    long long* timing;       // [grid][12] cycle counters per role (debug >= 0: always written, tiny)
     int single_pass;         // SPRL_EVALNET_PRECISION_FP16 (resident kernel): one fp16 MMA per product instead of the three of the hi/lo split
-    long long* trace;        // -DSPRL_EVALNET_TRACE builds: [phase][role: mma, epilogue X, epilogue Y][1 + 255 events] of CTA 0, clock << 12 | code
-    int debug;               // timing experiments only (SPRL_EVALNET_DEBUG): 1 skip lo pass, 3 no MMAs, 5 = 3 + no conv epilogue, 6 = MMAs but no conv epilogue
 };
 
 template <int C> inline int smem_bytes_for(int n_layers, int nst) {
-    return Width<C>::OFF_RING + nst * UNIT_SLOT + n_layers * C * 4 + (3 * nst + 2) * 8 + 16 + XCH_BYTES;
+    return Width<C>::OFF_RING + nst * UNIT_BYTES + n_layers * C * 4 + 16 + XCH_BYTES + (2 * nst + 1) * 8;
 }
 
 // ---- PTX wrappers ---------------------------------------------------------------------------
@@ -182,18 +152,8 @@ __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
 }
 __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
     uint32_t ok;
-#ifdef SPRL_EVALNET_TESTWAIT
-    asm volatile("{\n.reg .pred p;\nmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-#elif defined(SPRL_EVALNET_WAIT_HINT_NS)
-    // with a suspend-time hint the waiting warp sleeps in hardware until the phase completes (or the hint elapses)
-    // instead of polling: waiting warps were a third of the kernel's executed instructions
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\nselp.u32 %0, 1, 0, p;\n}"
-                 : "=r"(ok) : "r"(bar), "r"(parity), "r"((uint32_t)SPRL_EVALNET_WAIT_HINT_NS) : "memory");
-#else
     asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
                  : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-#endif
     return ok != 0;
 }
 // Bounded wait: a protocol bug must end as a reported error, never as a hung GPU.
@@ -261,9 +221,6 @@ __device__ __forceinline__ uint32_t map_to_cta(uint32_t addr, uint32_t rank) {
     uint32_t r;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
     return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-    if (elect_one()) asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
 __device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
     uint32_t ok;
@@ -344,10 +301,6 @@ __device__ __forceinline__ void split8(const float* x, uint4& hi, uint4& lo, flo
     hi = make_uint4(h[0], h[1], h[2], h[3]);
     lo = make_uint4(l[0], l[1], l[2], l[3]);
 }
-__device__ __forceinline__ void mma(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if (PAIR) umma_f16_pair(d_tmem, adesc, bdesc, idesc, accumulate);
-    else umma_f16(d_tmem, adesc, bdesc, idesc, accumulate);
-}
 // K-major, no swizzle: rows of a core matrix 16 B apart, 8-row groups SBO apart, K chunks (16 B) LBO apart
 __device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo, uint32_t sbo) {
     return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)((lbo >> 4) & 0x3fffu) << 16) |
@@ -383,27 +336,6 @@ __host__ __device__ inline int unit_bytes(const LayerGeom& g, int u) { return un
 // two zero rows first
 __device__ __forceinline__ int cell_slot(int m) { return m + 16; }
 
-// Per-role cycle counters (reported by sprl_evalnet_status when SPRL_EVALNET_TIMING is set) are compiled in only with
-// -DSPRL_EVALNET_TIMERS: a clock read costs tens of cycles and the MMA issuer runs ~200 of them per tile.
-#ifdef SPRL_EVALNET_TIMERS
-#define NOW() clock64()
-#else
-#define NOW() 0LL
-#endif
-// Event trace of one CTA pair's leader (resident kernel): every role keeps its events' count in a register and writes
-// (clock << 12 | stream << 8 | stage << 4 | kind) into its own region; dumped by sprl_evalnet_status.  kinds: 1 the MMA
-// warp may issue a stage (image barrier passed), 2 it has committed it, 3 the epilogue sees the accumulators, 4 it has
-// finished the stage (before its signal), 5 the next tile's input is written.
-#ifdef SPRL_EVALNET_TRACE
-#define TRACE_DECL(role) long long* trace_at = (net.trace && blockIdx.x == 0 && lane == 0) ? net.trace + ((long long)ph.index * 3 + (role)) * 256 : nullptr; int trace_n = 0;
-#define TRACE(s_, j_, kind_) do { if (trace_at && trace_n < 255) { trace_at[1 + trace_n] = (clock64() << 12) | ((long long)(s_) << 8) | ((long long)(j_) << 4) | (kind_); trace_n += 1; } } while (0)
-#define TRACE_END() do { if (trace_at) trace_at[0] = trace_n; } while (0)
-#else
-#define TRACE_DECL(role)
-#define TRACE(s_, j_, kind_) do { } while (0)
-#define TRACE_END() do { } while (0)
-#endif
-
 template <bool LINEAR, int C>
 __global__ void __launch_bounds__(THREADS, Width<C>::CTAS_PER_SM)
 k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsigned* __restrict__ d_rows,
@@ -414,9 +346,8 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_layers = net.n_layers, nst = net.nst;
     const uint32_t s_base = smem_u32(smem);
-    const int off_bias = W::OFF_RING + nst * UNIT_SLOT, off_bars = off_bias + n_layers * C * 4, off_tmem = off_bars + (3 * nst + 2) * 8;
+    const int off_bias = W::OFF_RING + nst * UNIT_BYTES, off_tmem = off_bias + n_layers * C * 4, off_bars = off_tmem + 16 + XCH_BYTES;
     const uint32_t bar_full = s_base + off_bars, bar_empty = bar_full + nst * 8, bar_acc = bar_empty + nst * 8;
-    const uint32_t bar_pfull = bar_acc + 8, bar_img = bar_pfull + nst * 8;      // pair mode, used in the leader: peer's half / image
     float* s_bias = reinterpret_cast<float*>(smem + off_bias);
     const long long n_tiles = LINEAR ? batch : (batch + 1) / 2;
     // every CTA of a cluster walks the same number of tiles (the multicast ring is shared);
@@ -433,24 +364,16 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
     for (int i = threadIdx.x; i < n_layers * C; i += THREADS)           // conv layers work in image units (x 2^ACT_SHIFT)
         s_bias[i] = net.bias[i] * (i < (n_layers - 1) * C ? ACT_SCALE : 1.0f);
     if (threadIdx.x == 0) {
-        for (int i = 0; i < nst; ++i) {
-            mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, PAIR ? 1 : CLUSTER); mbar_init(bar_pfull + 8 * i, 1);
-        }
+        for (int i = 0; i < nst; ++i) { mbar_init(bar_full + 8 * i, 1); mbar_init(bar_empty + 8 * i, CLUSTER); }
         mbar_init(bar_acc, 1);
-        mbar_init(bar_img, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     proxy_fence();
     __syncthreads();
     cluster_sync_all();                               // peers' barriers exist before anything is multicast
-    if (warp == MMA_WARP) {                           // pair mode: a collective of the two CTAs' MMA warps
-        if (PAIR) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(W::TMEM_COLS) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(W::TMEM_COLS) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+    if (warp == MMA_WARP) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_base + off_tmem), "r"(W::TMEM_COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
     tc_fence_before();
     __syncthreads();
@@ -461,13 +384,12 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
         // ===== weight producer =====
         if (lane == 0) {
             uint32_t s = 0, ph = 0;
-            long long t_wait = 0, t0 = NOW();
             for (long long tile = blockIdx.x; tile < tile_end; tile += gridDim.x) {
                 // Every tile needs the whole 1.2 MB of weights (shared memory has no room to keep
                 // them).  The CTAs of a cluster share ONE stream: each loads 1/CLUSTER of every unit
-                // and multicasts it to all.  Clusters read different replicas and walk the taps of a
-                // layer in different rotations (the accumulation order of taps is free) so that the
-                // chip is not pulling the same L2 lines at the same moment.
+                // and multicasts it to all.  Clusters read different replicas so that the chip is not
+                // pulling the same L2 lines at the same moment.  Every cluster walks the taps in the same
+                // order: a board's accumulation order, and so its outputs, must not depend on its CTA.
                 const unsigned char* layer_src = reinterpret_cast<const unsigned char*>(net.wunits) +
                                                  (size_t)(cluster_id % net.replicas) * net.wunits_bytes;
                 for (int layer = 0; layer < n_layers; ++layer) {
@@ -476,20 +398,14 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                     for (int u = 0; u < g.units_per_dy; ++u) dy_bytes += unit_bytes(g, u);
                     for (int h = 0; h < g.nh; ++h) {                     // output halves (128 channels), one after the other
                         for (int t = 0; t < g.ndy; ++t) {
-                            const int dyi = (t + ROTATE * cluster_id) % g.ndy;
-                            const unsigned char* src = layer_src + (size_t)dyi * dy_bytes;
+                            const unsigned char* src = layer_src + (size_t)t * dy_bytes;
                             for (int u = 0; u < g.units_per_dy; ++u) {
                                 const uint32_t bytes = (uint32_t)unit_bytes(g, u);
-                                { long long a = NOW(); mbar_wait(bar_empty + 8 * s, ph ^ 1u, net.error_flag, 1); t_wait += NOW() - a; }
+                                mbar_wait(bar_empty + 8 * s, ph ^ 1u, net.error_flag, 1);
                                 const uint32_t slice = bytes / CLUSTER;
-                                if (PAIR) {                                     // this CTA's half of the rows, kept to itself
-                                    mbar_expect_tx(bar_full + 8 * s, slice);
-                                    bulk_g2s(s_base + W::OFF_RING + s * UNIT_SLOT, src + crank * slice, slice, bar_full + 8 * s);
-                                } else {
-                                    mbar_expect_tx(bar_full + 8 * s, bytes);   // the whole unit: one slice from every CTA of the cluster
-                                    bulk_g2s_multicast(s_base + W::OFF_RING + s * UNIT_SLOT + crank * slice, src + crank * slice, slice,
-                                                       bar_full + 8 * s, CMASK);
-                                }
+                                mbar_expect_tx(bar_full + 8 * s, bytes);       // the whole unit: one slice from every CTA of the cluster
+                                bulk_g2s_multicast(s_base + W::OFF_RING + s * UNIT_BYTES + crank * slice, src + crank * slice, slice,
+                                                   bar_full + 8 * s, CMASK);
                                 src += bytes;
                                 if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
                             }
@@ -498,86 +414,59 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                     }
                 }
             }
-            if (net.timing) { net.timing[blockIdx.x * 12 + 8] = t_wait; net.timing[blockIdx.x * 12 + 9] = NOW() - t0; }
         }
         __syncwarp();
     } else if (warp == MMA_WARP) {
         // ===== MMA issuer (the whole warp runs the loop; one elected lane issues) =====
-        uint32_t s = 0, ph = 0, img_phase = 0;
-        const bool leader = !PAIR || crank == 0;
-        const uint32_t lead_pfull = PAIR ? map_to_cta(bar_pfull, 0) : 0u, lead_img = PAIR ? map_to_cta(bar_img, 0) : 0u;
-        long long t_bar = 0, t_full = 0, t_issue = 0, t_commit = 0, t0 = NOW();
+        uint32_t s = 0, ph = 0;
         for (long long tile = blockIdx.x; tile < tile_end; tile += gridDim.x) {
             for (int layer = 0; layer < n_layers; ++layer) {
                 const LayerGeom g = layer_geom<C>(layer, n_layers, net.in_ksteps);
-                { long long a = NOW(); named_bar(1, BAR1_THREADS); t_bar += NOW() - a; }   // the layer's input image is complete, the accumulators are drained
-                if (PAIR) {                                                      // ... in the peer CTA as well
-                    if (!leader) mbar_arrive_cluster(lead_img);
-                    else { long long a = NOW(); mbar_wait_cluster(bar_img, img_phase, net.error_flag, 4); img_phase ^= 1u; t_bar += NOW() - a; }
-                }
+                named_bar(1, BAR1_THREADS);                                      // the layer's input image is complete, the accumulators are drained
                 tc_fence_after();
-                const int n1 = g.ndx * g.n;                                      // output columns of one MMA
-                const int nb = PAIR ? n1 / 2 : n1;                               // weight rows held by this CTA
-                const uint32_t idesc = instr_desc_f16(PAIR ? 2 * TILE_M : TILE_M, n1);
-                const bool hi_pass = net.debug < 3 || net.debug == 6, lo_pass = net.debug != 1 && hi_pass;
-                const uint32_t b_lbo = (uint32_t)(2 * nb) * 16u, b_kstep = (2u * b_lbo) >> 4, b_lo_off = ((uint32_t)nb * 16u) >> 4;
+                const int n1 = g.ndx * g.n;                                      // output columns of one MMA = W_hi (and W_lo) rows of a unit
+                const uint32_t idesc = instr_desc_f16(TILE_M, n1);
+                const uint32_t b_lbo = (uint32_t)(2 * n1) * 16u, b_kstep = (2u * b_lbo) >> 4, b_lo_off = ((uint32_t)n1 * 16u) >> 4;
                 const uint64_t a_hi0 = smem_desc(s_base + W::OFF_AHI, CG_STRIDE, 128), a_lo0 = smem_desc(s_base + W::OFF_ALO, CG_STRIDE, 128);
                 const uint64_t b0 = smem_desc(s_base + W::OFF_RING, b_lbo, 128);
                 constexpr uint32_t A_KSTEP = (2u * CG_STRIDE) >> 4;
                 for (int h = 0; h < g.nh; ++h) {
                     const uint32_t d_main = tmem + h * 3 * CH;             // this half's accumulators
                     uint32_t acc = 0;                        // 0 for the very first MMA of the layer's half only
-                    for (int t = 0; t < g.ndy; ++t) {
-                        const int dyi = (t + ROTATE * cluster_id) % g.ndy;           // same order as the producer
-                        const int dy = g.ndy == 3 ? dyi - 1 : 0;
+                    for (int t = 0; t < g.ndy; ++t) {                        // same order as the producer
+                        const int dy = g.ndy == 3 ? t - 1 : 0;
                         // in 16-byte slots: two storage rows per board row, or one row of `cols` cells in the linear lattice
                         const uint32_t a_off = (uint32_t)(16 + (LINEAR ? net.cols : 16) * dy);
                         for (int u = 0; u < g.units_per_dy; ++u) {
                             const int nks = unit_ksteps(g, u);
-                            { long long a = NOW(); mbar_wait(bar_full + 8 * s, ph, net.error_flag, 2); t_full += NOW() - a; }
-                            if (PAIR && !leader) {                   // relay: the leader may read this CTA's half now
-                                mbar_arrive_cluster(lead_pfull + 8 * s);
-                                if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
-                                continue;
-                            }
-                            if (PAIR) { long long a = NOW(); mbar_wait_cluster(bar_pfull + 8 * s, ph, net.error_flag, 5); t_full += NOW() - a; }
+                            mbar_wait(bar_full + 8 * s, ph, net.error_flag, 2);
                             tc_fence_after();
-                            const long long t_i0 = NOW();
-                            const uint64_t bd = b0 + s * (UNIT_SLOT >> 4);
+                            const uint64_t bd = b0 + s * (UNIT_BYTES >> 4);
                             const uint64_t ah = a_hi0 + a_off + (uint32_t)(UNIT_KS * u) * A_KSTEP, al = a_lo0 + a_off + (uint32_t)(UNIT_KS * u) * A_KSTEP;
-                            if (hi_pass) {
-                                if (nks == UNIT_KS) {
+                            if (nks == UNIT_KS) {
 #pragma unroll
-                                    for (int ks = 0; ks < UNIT_KS; ++ks) {
-                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
-                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
-                                        if (lo_pass) mma(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
-                                        acc = 1;
-                                    }
-                                } else {
-                                    for (int ks = 0; ks < nks; ++ks) {
-                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
-                                        mma(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
-                                        if (lo_pass) mma(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
-                                        acc = 1;
-                                    }
+                                for (int ks = 0; ks < UNIT_KS; ++ks) {
+                                    umma_f16(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
+                                    umma_f16(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
+                                    umma_f16(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
+                                    acc = 1;
+                                }
+                            } else {
+                                for (int ks = 0; ks < nks; ++ks) {
+                                    umma_f16(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep, idesc, acc);
+                                    umma_f16(d_main, ah + ks * A_KSTEP, bd + ks * b_kstep + b_lo_off, idesc, 1u);
+                                    umma_f16(d_main, al + ks * A_KSTEP, bd + ks * b_kstep, idesc, 1u);
+                                    acc = 1;
                                 }
                             }
-                            const long long t_i1 = NOW();
-                            if (PAIR) umma_commit_pair(bar_empty + 8 * s);      // both producers may refill their halves
-                            else umma_commit_multicast(bar_empty + 8 * s, CMASK);   // every CTA's producer learns that this CTA is done with the unit
-                            t_issue += t_i1 - t_i0; t_commit += NOW() - t_i1;
+                            umma_commit_multicast(bar_empty + 8 * s, CMASK);   // every CTA's producer learns that this CTA is done with the unit
                             if (++s == (uint32_t)nst) { s = 0; ph ^= 1u; }
                         }
                     }
                 }
-                if (PAIR) { if (leader) umma_commit_pair(bar_acc); }        // the accumulators of this layer are complete, in both CTAs
-                else umma_commit(bar_acc);
+                umma_commit(bar_acc);                                  // the accumulators of this layer are complete
                 __syncwarp();
             }
-        }
-        if (lane == 0 && net.timing) {
-            net.timing[blockIdx.x * 12 + 0] = t_bar; net.timing[blockIdx.x * 12 + 1] = t_full; net.timing[blockIdx.x * 12 + 2] = NOW() - t0; net.timing[blockIdx.x * 12 + 3] = t_issue; net.timing[blockIdx.x * 12 + 10] = t_commit;
         }
     } else {
         // ===== epilogue warps: cell m = TMEM lane m =====
@@ -601,7 +490,6 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
         const float vmask = valid ? 1.0f : 0.0f, lmask = has_left ? 1.0f : 0.0f, rmask = has_right ? 1.0f : 0.0f;
         const int cells = net.rows * net.cols, planes = net.in_planes;
         uint32_t acc_phase = 0;
-        long long t_bar = 0, t_acc = 0, t_head = 0, t0 = NOW();
         // ---- input planes -> image (the reference's planes are 0/1, but any fp32 input is split).  The stem
         // has few input planes, so its vertical taps are folded into K: image channel dyi * planes + p of a
         // cell holds plane p of the cell one row above / at / below it, and the stem becomes a single-dy layer
@@ -623,11 +511,7 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
             const long long board = LINEAR ? tile : tile * 2 + b;
             for (int cg = half; cg < 2 * net.in_ksteps; cg += EPI_WARPS / 4) {
                 float v[KCH];
-#ifdef SPRL_EVALNET_NO_PREFETCH
-                if (false) {
-#else
                 if (cg == half) {
-#endif
 #pragma unroll
                     for (int j = 0; j < KCH; ++j) v[j] = vnext[j];
                 } else {
@@ -641,21 +525,16 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
             proxy_fence();
             for (int layer = 0; layer < n_layers; ++layer) {
                 tc_fence_before();
-                { long long a = NOW(); named_bar(1, BAR1_THREADS); t_bar += NOW() - a; }
-#ifndef SPRL_EVALNET_NO_PREFETCH
+                named_bar(1, BAR1_THREADS);
                 if (layer == n_layers - 1 && tile + gridDim.x < tile_end) load_planes(tile + gridDim.x, half, vnext);
-#endif
                 // accumulator -> image units for the conv layers (real units for the heads); exact powers of two (read
                 // before the wait below, which hides the load)
                 const float inv_scale = __ldg(net.inv_scale + layer) * (layer < n_layers - 1 ? ACT_SCALE : 1.0f);
-                { long long a = NOW(); mbar_wait(bar_acc, acc_phase, net.error_flag, 3); t_acc += NOW() - a; }
-                const long long t_layer = NOW();
+                mbar_wait(bar_acc, acc_phase, net.error_flag, 3);
                 acc_phase ^= 1u;
                 tc_fence_after();
                 const float* bias = s_bias + layer * C;
-                if (layer < n_layers - 1 && net.debug >= 5) {
-                    // timing experiment: no epilogue work
-                } else if (layer < n_layers - 1) {
+                if (layer < n_layers - 1) {
                     const bool add_res = layer > 0 && (layer & 1) == 0;      // second conv of a block
                     const bool save_res = (layer & 1) == 0;                  // block input of the next block
 #pragma unroll 1
@@ -718,26 +597,17 @@ k_evalnet(NetDev net, const float* __restrict__ in, long long batch, const unsig
                         for (int j = 0; j < 3; ++j)
                             if (j <= pc) dst[j * cells + cell] = fmaxf(v[j] * inv_scale + bias[j], 0.0f);
                     }
-                    t_head += NOW() - t_layer;
                 }
             }
         }
         if (mx > HALF_MAX) atomicExch(net.error_flag + 1, 1ULL);
-        if (threadIdx.x == 0 && net.timing) {
-            net.timing[blockIdx.x * 12 + 4] = t_bar; net.timing[blockIdx.x * 12 + 5] = t_acc; net.timing[blockIdx.x * 12 + 6] = t_head;
-            net.timing[blockIdx.x * 12 + 7] = NOW() - t0;
-        }
-    }
-    if (threadIdx.x == 0 && net.timing) {
-        // (only reached by the epilogue branch's thread 0)
     }
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();                               // no CTA leaves while peers may still signal its barriers
     if (warp == MMA_WARP) {
         tc_fence_after();
-        if (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(W::TMEM_COLS) : "memory");
-        else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(W::TMEM_COLS) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(W::TMEM_COLS) : "memory");
     }
 }
 
@@ -932,23 +802,20 @@ static int weight_shift(const std::vector<std::vector<float>>& b) {
 
 // appends the units of one vertical offset: b[dx][n][k] (n < n_pad rows, k < kk), per unit of <= UNIT_KS*16
 // input channels the layout [K chunk of 8][hi rows of every dx | lo rows of every dx][8 halfs]; weights x 2^shift
-// In pair mode a unit is [rows of CTA 0][rows of CTA 1], each with the layout above over its half of the rows
-// (row index = dx * n_pad + n): the two CTAs of a pair each load and hold one half.
 static void append_units(std::vector<unsigned short>& out, const std::vector<std::vector<float>>& b, int n_pad, int kk, int shift) {
-    const int ndx = (int)b.size(), rows = ndx * n_pad, parts = PAIR ? 2 : 1, rows_per = rows / parts;
+    const int ndx = (int)b.size(), rows = ndx * n_pad;
     for (int k0 = 0; k0 < kk; k0 += UNIT_KS * KSTEP_CH)
-        for (int h = 0; h < parts; ++h)
-            for (int kc = k0 / KCH; kc < std::min(kk, k0 + UNIT_KS * KSTEP_CH) / KCH; ++kc)
-                for (int part = 0; part < 2; ++part)
-                    for (int r = h * rows_per; r < (h + 1) * rows_per; ++r) {
-                        const int dx = r / n_pad, n = r - dx * n_pad;
-                        for (int j = 0; j < KCH; ++j) {
-                            const float w = std::ldexp(b[dx][(size_t)n * kk + kc * KCH + j], shift);
-                            const __half hi = __float2half_rn(w);
-                            const __half v = part == 0 ? hi : __float2half_rn(w - __half2float(hi));
-                            out.push_back(__half_as_ushort(v));
-                        }
+        for (int kc = k0 / KCH; kc < std::min(kk, k0 + UNIT_KS * KSTEP_CH) / KCH; ++kc)
+            for (int part = 0; part < 2; ++part)
+                for (int r = 0; r < rows; ++r) {
+                    const int dx = r / n_pad, n = r - dx * n_pad;
+                    for (int j = 0; j < KCH; ++j) {
+                        const float w = std::ldexp(b[dx][(size_t)n * kk + kc * KCH + j], shift);
+                        const __half hi = __float2half_rn(w);
+                        const __half v = part == 0 ? hi : __float2half_rn(w - __half2float(hi));
+                        out.push_back(__half_as_ushort(v));
                     }
+                }
 }
 
 // Resident format (k_evalnet_resident): the weights of one vertical offset held by CTA `h` of a pair,
@@ -1003,7 +870,9 @@ struct sprl_evalnet {
     float* act = nullptr;          // [act_cap_tiles][RB_ACT_TILE_FLOATS]
     int64_t act_cap_tiles = 0;
     int path = 0;                  // SPRL_EVALNET_PATH_*: 0 auto (resident when the network fits), 1 streaming, 2 resident
-    int max_ctas = 0;              // experiments (SPRL_EVALNET_MAX_CTAS): caps the resident kernel's grid, leaving SMs to a concurrent search launch
+    int max_ctas = 0;              // SPRL_EVALNET_MAX_CTAS, read at create: caps the resident kernel's grid.  Set to 2, one CTA pair
+                                   // walks every quad of the batch (the test of the pairs' quad loop); larger caps leave SMs to a
+                                   // concurrent search launch (tools/explore_overlap.py)
     // First call allocates; later calls (a new generation's weights) overwrite in place, so device
     // pointers captured in a CUDA graph stay valid.
     template <typename T> int upload(const std::vector<T>& h, const T** out) {
@@ -1155,7 +1024,6 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
                     }
                     rbw.resize(start + (size_t)ph.w_bytes / 2, 0);
                 }
-                ph.index = (int)i;
                 phases.push_back(ph);
             }
             for (size_t i = 0; i < phases.size(); ++i) phases[i].w = reinterpret_cast<const unsigned char*>(w_at[i] * 2);   // offsets until the upload below
@@ -1177,23 +1045,7 @@ static int pack_and_upload(sprl_evalnet* e, const sprl_network_params* p) {
     for (int r = 1; r < REPLICAS; ++r) std::copy(units.begin(), units.begin() + one, units.begin() + r * one);
     e->dev.wunits_bytes = (long long)(one * sizeof(unsigned short));
     e->dev.replicas = REPLICAS;
-    e->dev.debug = getenv("SPRL_EVALNET_DEBUG") ? atoi(getenv("SPRL_EVALNET_DEBUG")) : 0;
-#ifdef SPRL_EVALNET_TRACE
-    if (getenv("SPRL_EVALNET_TRACE") && !e->dev.trace) {
-        std::vector<long long> z(16 * 3 * 256, 0);
-        const long long* tp = nullptr;
-        if (!e->upload(z, &tp)) e->dev.trace = const_cast<long long*>(tp);
-    }
-#endif
-#ifdef SPRL_EVALNET_TIMERS        // per-role cycle counters: only in builds that compile the clock reads in
-    if (getenv("SPRL_EVALNET_TIMING") && !e->dev.timing) {
-        std::vector<long long> z(1024 * 12, 0);
-        const long long* tp = nullptr;
-        if (!e->upload(z, &tp)) e->dev.timing = const_cast<long long*>(tp);
-    }
-#endif
     e->dev.nst = MAX_NST;
-    if (getenv("SPRL_EVALNET_NST")) e->dev.nst = std::max(2, std::min(MAX_NST, atoi(getenv("SPRL_EVALNET_NST"))));   // experiments
     while (e->dev.nst > 2 && stream_smem_bytes(C, L, e->dev.nst) > stream_max_smem(C)) e->dev.nst -= 1;
     int rc = e->upload(units, &e->dev.wunits);
     if (!rc) rc = e->upload(head_w, &e->dev.head_w);
@@ -1267,7 +1119,6 @@ int sprl_evalnet_create(int device, const sprl_network_params* params, sprl_eval
     if (prop.major != 10) { delete e; return fail(SPRL_E_NOGPU, "the tcgen05 evaluator needs an sm_100a device (found sm_%d%d)", prop.major, prop.minor); }
     e->sm_count = prop.multiProcessorCount;
     if (getenv("SPRL_EVALNET_MAX_CTAS")) e->max_ctas = atoi(getenv("SPRL_EVALNET_MAX_CTAS"));
-    if (getenv("SPRL_EVALNET_PATH")) e->path = atoi(getenv("SPRL_EVALNET_PATH"));      // experiments: 1 streaming, 2 resident
     err = cudaFuncSetAttribute(k_evalnet<false, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<CH>::MAX_SMEM);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet<true, CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<CH>::MAX_SMEM);
     if (err == cudaSuccess) err = cudaFuncSetAttribute(k_evalnet<false, WIDE_CH>, cudaFuncAttributeMaxDynamicSharedMemorySize, Width<WIDE_CH>::MAX_SMEM);
@@ -1406,33 +1257,6 @@ int sprl_evalnet_status(sprl_evalnet* e, uint64_t* launches) {
     if (err != cudaSuccess) return fail(SPRL_E_CUDA, "evaluator kernel failed: %s", cudaGetErrorString(err));
     if (flag[0]) return fail(SPRL_E_CUDA, "evaluator kernel timed out on a pipeline barrier (code %llx)", flag[0]);
     if (flag[1]) return fail(SPRL_E_STATE, "an input or activation exceeded %.0f, the range of the fp16-split evaluator; its outputs were clamped", HALF_MAX / ACT_SCALE);
-    if (e->dev.timing) {
-        std::vector<long long> t(12 * 1024);
-        cudaMemcpy(t.data(), e->dev.timing, t.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        const bool res = !e->phases.empty() && e->path != SPRL_EVALNET_PATH_STREAMING;
-        for (int b = 0; b < (res ? 160 * (int)e->phases.size() : 2); b += (res ? 160 : 1))       // streaming kernel: mma {bar, full, total, issue} epi {bar, acc, heads, total} producer {empty, total} mma commit;
-                                          // resident kernel: mma {wait img, -, total} epi {wait acc X, Y, total X, Y}
-            fprintf(stderr, "[evalnet timing, CTA %d, last launch] %lld %lld %lld %lld | %lld %lld %lld %lld | %lld %lld %lld\n",
-                    b, t[b * 12 + 0], t[b * 12 + 1], t[b * 12 + 2], t[b * 12 + 3], t[b * 12 + 4], t[b * 12 + 5], t[b * 12 + 6], t[b * 12 + 7], t[b * 12 + 8], t[b * 12 + 9], t[b * 12 + 10]);
-    }
-#ifdef SPRL_EVALNET_TRACE
-    if (e->dev.trace) {
-        std::vector<long long> t(16 * 3 * 256);
-        cudaMemcpy(t.data(), e->dev.trace, t.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        static const char* kinds[] = { "?", "mma_may_issue", "mma_committed", "epi_acc_ready", "epi_stage_done", "epi_next_input_written" };
-        for (size_t phx = 0; phx < e->phases.size() && phx < 16; ++phx) {
-            std::vector<long long> ev;
-            for (int role = 0; role < 3; ++role) {
-                const long long* r = t.data() + (phx * 3 + role) * 256;
-                for (long long i = 0; i < r[0] && i < 255; ++i) ev.push_back(r[1 + i]);
-            }
-            std::sort(ev.begin(), ev.end());
-            fprintf(stderr, "== phase %zu: %zu events\n", phx, ev.size());
-            for (long long x : ev)
-                fprintf(stderr, "%8lld  %-22s stream %lld stage %lld\n", (x >> 12) - (ev[0] >> 12), kinds[std::min<long long>(x & 15, 5)], (x >> 8) & 15, (x >> 4) & 15);
-        }
-    }
-#endif
     if (launches) *launches = e->launches;
     return SPRL_OK;
 }

@@ -62,7 +62,6 @@ struct RbPhase {
     const unsigned char* w;      // [2][w_bytes]: the resident weights of CTA rank 0 / rank 1 (each holds half of the rows)
     int w_bytes;                 // per CTA, a multiple of 128
     float* act;                  // [tiles][16 channel quads][128 cells][4]: activations between phases, image units, in place
-    int index;                   // position of the phase in the forward (timing slots)
 };
 // linear lattice (boards wider than 8, one per tile): Z_-1 / Z_+1 of a warp's edge lanes for its neighbour warps,
 // [stream][channel half][double buffer][warp of the quarter][left | right][16 values]
@@ -134,8 +133,6 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
         if (crank == 0) {
             uint32_t img_phase = 0u;                                             // bit s: parity of stream s's next wait
             const bool split = net.single_pass == 0;                             // (SPRL_EVALNET_PRECISION_FP16: hi x hi only)
-            TRACE_DECL(0)
-            long long t_wait = 0, t0 = NOW();
             constexpr uint32_t A_KSTEP = (2u * RB_CG_STRIDE) >> 4;
             for (long long quad = pair; quad < n_quads; quad += n_pairs) {
                 for (int j = 0; j < ph.n_stages; ++j) {
@@ -146,10 +143,9 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
                     const uint64_t b0 = smem_desc(s_base + RB_OFF_W + S.w_off, b_lbo, 128);
 #pragma unroll 1
                     for (int s = 0; s < RB_STREAMS; ++s) {
-                        { long long a = NOW(); mbar_wait_cluster(bar_img + 8 * s, (img_phase >> s) & 1u, net.error_flag, 10 + s); t_wait += NOW() - a; }
+                        mbar_wait_cluster(bar_img + 8 * s, (img_phase >> s) & 1u, net.error_flag, 10 + s);
                         img_phase ^= 1u << s;
                         tc_fence_after();
-                        TRACE(s, j, 1);
                         const uint64_t a_hi0 = smem_desc(s_base + (2 * s) * RB_IMG_BYTES, RB_CG_STRIDE, 128);
                         const uint64_t a_lo0 = smem_desc(s_base + (2 * s + 1) * RB_IMG_BYTES, RB_CG_STRIDE, 128);
                         const uint32_t d_tmem = tmem + (uint32_t)(s * RB_STREAM_COLS);
@@ -171,12 +167,9 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
                         }
                         umma_commit_pair(bar_acc + 8 * s);                      // both CTAs' epilogue groups of stream s
                         __syncwarp();
-                        TRACE(s, j, 2);
                     }
                 }
             }
-            if (lane == 0 && net.timing) { long long* tm = net.timing + (ph.index * 160 + blockIdx.x) * 12; tm[0] = t_wait; tm[2] = NOW() - t0; }
-            TRACE_END();
         }
     } else {
         // ===== epilogue group of stream s: cell m = TMEM lane m =====
@@ -201,7 +194,6 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
         const float vmask = valid ? 1.0f : 0.0f, lmask = c > 0 ? 1.0f : 0.0f, rmask = c + 1 < net.cols ? 1.0f : 0.0f;
         const int cells = net.rows * net.cols, planes = net.in_planes;
         uint32_t acc_phase = 0;
-        long long t_acc = 0, t0 = NOW();
         // "my part of stream s's image is written and I am done reading its accumulators", to the leader's MMA warp
         auto signal = [&]() {
             proxy_fence();
@@ -272,10 +264,6 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
         if (planes_in) load_planes(tile0, half, vnext);
         mbar_wait(bar_w, 0u, net.error_flag, 20);                   // (the leader's MMAs read both CTAs' weights: every arrival below implies them)
         float xin[16];
-        TRACE_DECL(w8 == 0 ? 1 + s : 3)
-#ifdef SPRL_EVALNET_TRACE
-        if (w8 != 0) trace_at = nullptr;
-#endif
         // ---- input of the first tile; every later tile's input is written by the last stage's epilogue of the tile before ----
         if (planes_in) put_planes(tile0);
         else {
@@ -303,10 +291,9 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
                     if (planes_in) load_planes(next, half, vnext);
                     else load_acts(next, 2 * half, xin);
                 }
-                { long long a = NOW(); mbar_wait(bar_acc + 8 * s, acc_phase, net.error_flag, 30 + s); t_acc += NOW() - a; }
+                mbar_wait(bar_acc + 8 * s, acc_phase, net.error_flag, 30 + s);
                 acc_phase ^= 1u;
                 tc_fence_after();
-                TRACE(s, j, 3);
                 // the image is free from here on in the last stage: its MMAs are complete and its output does not go there
                 if (feed && planes_in) put_planes(next);
                 const float* bias = s_bias + j * CH;
@@ -402,14 +389,11 @@ k_evalnet_resident(NetDev net, RbPhase ph, const float* __restrict__ in, long lo
                     }
                 };
                 if (heads_first) finish_heads();
-                TRACE(s, j, feed ? 5 : 4);
                 if (j < last_stage || has_next) signal();
                 if (S.heads && !heads_first) finish_heads();
             }
         }
         if (mx > HALF_MAX) atomicExch(net.error_flag + 1, 1ULL);
-        TRACE_END();
-        if (w8 == 0 && lane == 0 && net.timing) { long long* tm = net.timing + (ph.index * 160 + blockIdx.x) * 12; tm[4 + s] = t_acc; tm[6 + s] = NOW() - t0; }
     }
     tc_fence_before();
     __syncthreads();

@@ -1003,14 +1003,8 @@ struct TreeWarp {
 };
 
 // ---- kernels -------------------------------------------------------------------------------------
-#ifndef SPRL_SEARCH_WARPS_PER_BLOCK
-#define SPRL_SEARCH_WARPS_PER_BLOCK 1
-#endif
-constexpr int WARPS_PER_BLOCK = SPRL_SEARCH_WARPS_PER_BLOCK;      // 1: one tree per block, a finished tree frees its slot at once
-#ifndef SPRL_SEARCH_BLOCKS_PER_SM
-#define SPRL_SEARCH_BLOCKS_PER_SM 32
-#endif
-constexpr int MIN_BLOCKS_PER_SM = SPRL_SEARCH_BLOCKS_PER_SM;      // 32: 64 registers per thread -> 32 resident warps per SM
+constexpr int WARPS_PER_BLOCK = 1;          // 1: one tree per block, a finished tree frees its slot at once
+constexpr int MIN_BLOCKS_PER_SM = 32;       // 32: 64 registers per thread -> 32 resident warps per SM
 
 template <class G>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32) k_begin(EngineParams p) {

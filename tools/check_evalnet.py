@@ -34,7 +34,7 @@ el, evv = (lg.cpu().double() - ref_l).abs().max().item(), (v.cpu().double() - re
 fl, fv = (f32_l.double() - ref_l).abs().max().item(), (f32_v.double() - ref_v).abs().max().item()
 print(f"B={B} blocks={blocks}: max|dlogit| vs fp64: ours {el:.3e} (torch fp32 CPU {fl:.3e}); max|dvalue| ours {evv:.3e} (torch {fv:.3e}); "
       f"logit scale {ref_l.abs().max().item():.3f}", flush=True)
-if (el > 1e-4 or evv > 1e-4) and not os.environ.get('SPRL_EVALNET_DEBUG'):
+if el > 1e-4 or evv > 1e-4:
     bad = (lg.cpu().double() - ref_l).abs().amax(1)
     print("worst boards:", bad.topk(min(8, B)).indices.tolist(), bad.topk(min(8, B)).values.tolist())
     print("ours[0,:8]", lg[0, :8].tolist(), "\nref [0,:8]", ref_l[0, :8].tolist())
