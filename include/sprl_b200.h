@@ -159,6 +159,20 @@ int sprl_begin_iteration(sprl_engine* e, uint64_t first_game, int64_t num_games)
  * first_game = base + r and stride = world.  Default stride 1. */
 int sprl_set_game_stride(sprl_engine* e, uint64_t stride);
 
+/* Opening lines for the games / trees the NEXT sprl_begin_iteration, sprl_match_begin or sprl_begin_trees starts.
+ * Line i = h_actions[h_offsets[i] .. h_offsets[i+1]-1], a sequence of actions from the start position; n_lines = 0
+ * turns openings off (the default).  Self-play games and step-wise trees with stream id t start from line t % n_lines;
+ * match games from line (t / 2) % n_lines, so that ids 2k and 2k+1 play one line with the colours swapped (agent t % 2
+ * still plays Player ZERO).  Starting from a line means exactly: the tree is built at the start position and advanced
+ * through the line (as sprl_advance does) before any search.  The line draws no random numbers, its positions are the
+ * game's history (network inputs, sample planes, Go's superko), and the decision node starts unsearched.  Samples, move
+ * statistics, move counts (sprl_iteration_counts, sprl_move_stats, sprl_match_results, sprl_stats.moves) cover the
+ * searched moves only; the temperature of self-play counts searched moves; the outcome is that of the finished game.
+ * Every line is replayed once on the device when it is set.  Fails with SPRL_E_INVALID for an illegal action or a line
+ * that reaches a terminal position (message names line and ply), SPRL_E_STATE while an iteration / match / set of
+ * trees is open (still has a game or tree playing); the previous lines then stay in force. */
+int sprl_set_openings(sprl_engine* e, int64_t n_lines, const int64_t* h_offsets, const int32_t* h_actions);
+
 /* Enqueues one search launch: apply the evaluations of the previous launch, finish
  * moves whose traversal budget is spent (sample, re-root, compact), then run the next
  * searchAndGetLeaves batch of every live tree.  Asynchronous, capturable in a CUDA graph. */

@@ -21,7 +21,7 @@ EVALNET_PRECISION_FP32_SPLIT, EVALNET_PRECISION_FP16 = 0, 1
 EXPORTS = [
     "sprl_last_error", "sprl_device_count", "sprl_game_info_get", "sprl_env_step", "sprl_env_line", "sprl_env_rollout",
     "sprl_env_perft", "sprl_default_config", "sprl_create", "sprl_destroy", "sprl_set_stream",
-    "sprl_bind_eval_buffers", "sprl_eval_batch", "sprl_eval_rows", "sprl_set_game_stride", "sprl_begin_iteration", "sprl_round", "sprl_poll",
+    "sprl_bind_eval_buffers", "sprl_eval_batch", "sprl_eval_rows", "sprl_set_game_stride", "sprl_set_openings", "sprl_begin_iteration", "sprl_round", "sprl_poll",
     "sprl_run_iteration", "sprl_iteration_counts", "sprl_collect_samples", "sprl_collect_samples_device", "sprl_stream_samples", "sprl_stream_info",
     "sprl_match_begin", "sprl_run_match", "sprl_match_results", "sprl_begin_trees", "sprl_search", "sprl_search_batch",
     "sprl_apply_evaluations", "sprl_root_stats", "sprl_advance", "sprl_move_stats", "sprl_debug_check_guards", "sprl_get_stats", "sprl_reset_stats", "sprl_write_npy_f32",
@@ -101,6 +101,7 @@ def load():
     lib.sprl_bind_eval_buffers.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.sprl_eval_rows.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
     lib.sprl_set_game_stride.argtypes = [C.c_void_p, C.c_uint64]
+    lib.sprl_set_openings.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     lib.sprl_begin_iteration.argtypes = [C.c_void_p, C.c_uint64, C.c_int64]
     lib.sprl_round.argtypes = [C.c_void_p]
     lib.sprl_poll.argtypes = [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]

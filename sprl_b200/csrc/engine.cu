@@ -20,6 +20,8 @@ void search_launch_tree_stats(int game, const EngineParams& p, int n, float* N, 
                               signed char* te, signed char* wi, int* tr, signed char* mk, int* qu, cudaStream_t s);
 void search_launch_tree_advance(int game, const EngineParams& p, int n, const int* actions, cudaStream_t s);
 int search_header_units(int game);
+void env_launch_lines(int game, int n_lines, const long long* off, const int* actions, PosRec* rec, u64* hist, int* bad,
+                      cudaStream_t s);
 }  // namespace sprl
 
 using namespace sprl;
@@ -39,6 +41,10 @@ struct sprl_engine {
     bool stepwise = false;          // the open iteration is a set of step-wise trees (sprl_begin_trees)
     int step_sims = 0;
     bool step_single = false;
+    // opening lines of the games the next begin starts (sprl_set_openings; IterParams describes the layout)
+    int64_t n_lines = 0;
+    long long* d_open_off = nullptr;
+    PosRec* d_open_rec = nullptr;
     unsigned char* d_tree_io = nullptr;     // staging of sprl_root_stats / sprl_advance, sized for num_slots trees
     // Streamed sample output (sprl_stream_samples): finished games are embedded and copied to the caller's (pinned) host
     // arrays while the others still play.  Two copy streams, each with its own staging buffers of `rows` sample rows.
@@ -87,6 +93,15 @@ struct sprl_engine {
         device_bytes += bytes + 2 * GUARD;
         *out = (T*)(base + GUARD);
         return SPRL_OK;
+    }
+    // frees one pool taken by alloc()
+    void release(void* ptr) {
+        if (!ptr) return;
+        unsigned char* base = (unsigned char*)ptr - GUARD;
+        for (size_t i = 0; i < pools.size(); ++i)
+            if (pools[i].base == base) { device_bytes -= pools[i].bytes + 2 * GUARD; pools.erase(pools.begin() + i); break; }
+        allocations.erase(std::remove(allocations.begin(), allocations.end(), (void*)base), allocations.end());
+        cudaFree(base);
     }
     void free_all() {
         for (void* q : allocations) cudaFree(q);
@@ -157,6 +172,7 @@ static int push_iter_params(sprl_engine* e) {
     it.num_games = e->p.num_games; it.first_game = e->p.first_game; it.game_stride = e->p.game_stride; it.q_half = e->p.q_half;
     it.stepwise = e->stepwise ? 1 : 0; it.step_sims = e->step_sims; it.step_single = e->step_single ? 1 : 0;
     it.agent[0] = e->match.agent[0]; it.agent[1] = e->match.agent[1];
+    it.n_lines = e->n_lines; it.open_off = e->d_open_off; it.open_rec = e->d_open_rec;
     cudaError_t err = cudaMemcpyAsync(e->d_iter, &it, sizeof(it), cudaMemcpyHostToDevice, e->stream);   // pageable source: staged before the call returns
     if (err != cudaSuccess) { e->failed = true; return fail(SPRL_E_CUDA, "cudaMemcpyAsync of the iteration parameters failed: %s", cudaGetErrorString(err)); }
     return SPRL_OK;
@@ -274,6 +290,7 @@ int sprl_create(const sprl_config* cfg, sprl_engine** out) {
     if (!rc) rc = e->alloc(&p.rec_player, MG * MM, true);
     if (!rc) rc = e->alloc(&p.rec_pdf, MG * MM * A, false);
     if (!rc) rc = e->alloc(&p.rec_moves, MG, true);
+    if (!rc) rc = e->alloc(&p.rec_open, MG, true);
     if (!rc) rc = e->alloc(&p.rec_winner, MG, true);
     if (!rc) rc = e->alloc(&p.rec_draws, MG, true);
     if (!rc) rc = e->alloc(&p.counters, 4, true);
@@ -336,6 +353,76 @@ int sprl_eval_rows(sprl_engine* e, const uint32_t** d_rows) {
 }
 
 int64_t sprl_eval_batch(const sprl_engine* e) { return e ? (int64_t)e->cfg.num_slots * e->cfg.max_queue : 0; }
+
+int sprl_set_openings(sprl_engine* e, int64_t n_lines, const int64_t* h_offsets, const int32_t* h_actions) {
+    NvtxRange nvtx_range("sprl_set_openings");
+    ENGINE_CHECK(e);
+    if (n_lines < 0 || n_lines > (1 << 30)) return fail(SPRL_E_INVALID, "n_lines = %lld is out of range", (long long)n_lines);
+    if (n_lines > 0 && !h_offsets) return fail(SPRL_E_INVALID, "null offsets");
+    if (e->iteration_open) {
+        // slots start games from the table until the last game has started: it changes only when no game is playing
+        unsigned long long c[4] = { 0, 0, 0, 0 };
+        ENGINE_CUDA(e, cudaMemcpyAsync(c, e->p.counters, sizeof(c), cudaMemcpyDeviceToHost, e->stream));
+        ENGINE_CUDA(e, cudaStreamSynchronize(e->stream));
+        if (e->active_slots - (int64_t)c[0] - (int64_t)c[1] > 0)
+            return fail(SPRL_E_STATE, "openings cannot change while an iteration, a match or a set of step-wise trees is still playing");
+    }
+    int64_t total = 0;
+    if (n_lines > 0) {
+        if (h_offsets[0] != 0) return fail(SPRL_E_INVALID, "h_offsets[0] must be 0");
+        for (int64_t i = 0; i < n_lines; ++i)
+            if (h_offsets[i + 1] < h_offsets[i]) return fail(SPRL_E_INVALID, "h_offsets must not decrease (line %lld)", (long long)i);
+        total = h_offsets[n_lines];
+        if (total > (1 << 30)) return fail(SPRL_E_INVALID, "the lines hold %lld actions, more than %d", (long long)total, 1 << 30);
+        if (total > 0 && !h_actions) return fail(SPRL_E_INVALID, "null actions");
+    }
+    // every line is replayed once, on the device; the old table stays in use until the new one has been checked
+    long long* d_off = nullptr;
+    PosRec* d_rec = nullptr;
+    if (n_lines > 0) {
+        int rc = e->alloc(&d_off, (size_t)n_lines + 1, false);
+        if (!rc) rc = e->alloc(&d_rec, (size_t)(total + n_lines), false);
+        if (rc) { e->release(d_off); return rc; }
+        DeviceBuf<int> d_act, d_bad;
+        DeviceBuf<u64> d_hist;
+        cudaError_t err = d_act.alloc((size_t)std::max<int64_t>(total, 1));
+        if (err == cudaSuccess) err = d_bad.alloc((size_t)n_lines);
+        if (err == cudaSuccess) err = d_hist.alloc((size_t)std::max<int64_t>(total, 1) * 2 * e->words);
+        if (err == cudaSuccess) err = cudaMemcpyAsync(d_off, h_offsets, ((size_t)n_lines + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, e->stream);
+        if (err == cudaSuccess && total > 0) err = cudaMemcpyAsync(d_act.p, h_actions, (size_t)total * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream);
+        if (err == cudaSuccess) {
+            env_launch_lines(e->cfg.game, (int)n_lines, d_off, d_act.p, d_rec, d_hist.p, d_bad.p, e->stream);
+            e->launches += 1;
+            err = cudaGetLastError();
+        }
+        std::vector<int> bad((size_t)n_lines);
+        std::vector<PosRec> rec((size_t)(total + n_lines));
+        if (err == cudaSuccess) err = cudaMemcpyAsync(bad.data(), d_bad.p, bad.size() * sizeof(int), cudaMemcpyDeviceToHost, e->stream);
+        if (err == cudaSuccess) err = cudaMemcpyAsync(rec.data(), d_rec, rec.size() * sizeof(PosRec), cudaMemcpyDeviceToHost, e->stream);
+        if (err == cudaSuccess) err = cudaStreamSynchronize(e->stream);
+        if (err != cudaSuccess) {
+            e->failed = true;
+            return fail(SPRL_E_CUDA, "replay of the opening lines failed: %s", cudaGetErrorString(err));
+        }
+        for (int64_t i = 0; i < n_lines; ++i) {
+            const int64_t ply = bad[i] >= 0 ? bad[i] : h_offsets[i + 1] - h_offsets[i];     // where the replay stopped
+            int rc = SPRL_OK;
+            if (rec[(size_t)(h_offsets[i] + i + ply)].terminal)
+                rc = fail(SPRL_E_INVALID, "opening line %lld reaches a terminal position at ply %lld: a game must have a move left to search",
+                          (long long)i, (long long)ply);
+            else if (bad[i] >= 0)
+                rc = fail(SPRL_E_INVALID, "opening line %lld: action %d at ply %lld is not legal in the position it is played in",
+                          (long long)i, h_actions[h_offsets[i] + ply], (long long)ply);
+            if (rc) { e->release(d_rec); e->release(d_off); return rc; }
+        }
+    }
+    e->release(e->d_open_rec);
+    e->release(e->d_open_off);
+    e->d_open_off = d_off;
+    e->d_open_rec = d_rec;
+    e->n_lines = n_lines;
+    return SPRL_OK;
+}
 
 int sprl_begin_iteration(sprl_engine* e, uint64_t first_game, int64_t num_games) {
     NvtxRange nvtx_range("sprl_begin_iteration");
@@ -737,9 +824,12 @@ int sprl_move_stats(sprl_engine* e, int64_t cap_moves, float* h_N, float* h_W, f
     if (n_moves) *n_moves = moves;
     if (moves > cap_moves) return fail(SPRL_E_CAPACITY, "%lld moves do not fit the caller's capacity %lld", (long long)moves, (long long)cap_moves);
     const size_t A = (size_t)e->gi.actions, MM = (size_t)e->p.max_moves;
+    std::vector<int> open((size_t)e->num_games);         // a game's searched moves are recorded after its opening's plies
+    ENGINE_CUDA(e, cudaMemcpyAsync(open.data(), e->p.rec_open, open.size() * sizeof(int), cudaMemcpyDeviceToHost, e->stream));
+    ENGINE_CUDA(e, cudaStreamSynchronize(e->stream));
     int64_t at = 0;
     for (int64_t g = 0; g < e->num_games; ++g) {
-        size_t m = (size_t)e->h_moves[g], src = (size_t)g * MM;
+        size_t m = (size_t)e->h_moves[g], src = (size_t)g * MM + (size_t)open[g];
         if (m == 0) continue;
         if (h_N) ENGINE_CUDA(e, cudaMemcpyAsync(h_N + at * A, e->p.rec_N + src * A, m * A * 4, cudaMemcpyDeviceToHost, e->stream));
         if (h_W) ENGINE_CUDA(e, cudaMemcpyAsync(h_W + at * A, e->p.rec_W + src * A, m * A * 4, cudaMemcpyDeviceToHost, e->stream));

@@ -36,38 +36,6 @@ int use_device(int device) {
     return SPRL_OK;
 }
 
-// ---- compact position record exchanged with the host ----------------------------
-struct alignas(16) PosRec {
-    u64 b[4];       // b0 words, then b1 words (W each; unused = 0)
-    u64 legal[2];
-    int action;     // action taken from this position (-1: none)
-    unsigned char player, pass_legal, terminal, winner;
-    u32 parent;     // perft: index of the parent in the previous level
-    u32 pad;
-};
-
-template <class G>
-__host__ __device__ inline void pos_to_rec(const typename G::P& p, PosRec& r) {
-    for (int i = 0; i < 2; ++i) {
-        r.b[i] = i < G::W ? p.b[0].word(i) : 0;
-        r.b[2 + i] = i < G::W ? p.b[1].word(i) : 0;
-        r.legal[i] = i < G::W ? p.legal.word(i) : 0;
-    }
-    r.player = p.player; r.pass_legal = p.pass_legal; r.terminal = p.terminal; r.winner = p.winner;
-    r.action = p.action | (p.depth << 8);   // perft keeps action/depth here; rollouts overwrite
-    r.parent = 0; r.pad = 0;
-}
-template <class G>
-__host__ __device__ inline void rec_to_pos(const PosRec& r, typename G::P& p) {
-    for (int i = 0; i < G::W; ++i) {
-        p.b[0].set_word(i, r.b[i]);
-        p.b[1].set_word(i, r.b[2 + i]);
-        p.legal.set_word(i, r.legal[i]);
-    }
-    p.player = r.player; p.pass_legal = r.pass_legal; p.terminal = r.terminal; p.winner = r.winner;
-    p.action = (unsigned char)(r.action & 0xff); p.depth = (unsigned short)(r.action >> 8);
-}
-
 // History of the boards of one line of play, oldest first: [count][2*W] words.
 template <int W>
 struct LineHist {
@@ -106,33 +74,50 @@ __global__ void k_env_step(int64_t n, const u64* __restrict__ b0, const u64* __r
     pos_to_rec<G>(nx, out[i]);
 }
 
-// ---- one line of play from the start position (a chain of GameNode::getAddChild calls, games/GameNode.hpp:96-110) ----
-// One thread: the line is sequential.  rec[k] = the position after k actions; for Go the line is the history of the
-// positional-superko rule.  *bad = index of the first action that is not legal where it is played (or -1).
+// ---- lines of play from the start position (chains of GameNode::getAddChild calls, games/GameNode.hpp:96-110) ----
+// One thread per line: a line is sequential.  Line i = actions[off[i] .. off[i+1]-1]; rec[off[i] + i + k] = the position
+// after k of its actions, k = 0 .. its length (rec_to_pos restores each exactly, depth included); for Go the line is the
+// history of the positional-superko rule, kept in hist[off[i] ..].  bad[i] = index of the first action of line i that is
+// not legal where it is played (or -1).
 template <class G>
-__global__ void k_env_line(int n_actions, const int* __restrict__ actions, PosRec* __restrict__ rec,
-                           u64* __restrict__ hist /* [n_actions + 1][2W] */, int* __restrict__ bad) {
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+__global__ void k_env_lines(int n_lines, const long long* __restrict__ off, const int* __restrict__ actions,
+                            PosRec* __restrict__ rec, u64* __restrict__ hist /* [total actions][2W] */, int* __restrict__ bad) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_lines) return;
+    const long long a0 = off[i];
+    const int n_actions = (int)(off[i + 1] - a0);
+    const int* act = actions + a0;
+    PosRec* r = rec + a0 + i;
+    u64* h = hist + (size_t)a0 * 2 * G::W;
     typename G::P cur, nx;
     G::start(cur);
-    *bad = -1;
+    bad[i] = -1;
     for (int k = 0;; ++k) {
-        PosRec r;
-        pos_to_rec<G>(cur, r);
-        r.action = k < n_actions ? actions[k] : -1;
-        rec[k] = r;
+        pos_to_rec<G>(cur, r[k]);
         if (k == n_actions) break;
-        const int a = actions[k];
+        const int a = act[k];
         const bool legal = !cur.terminal && a >= 0 && a < G::ACTIONS &&
                            ((G::HAS_PASS && a == G::CELLS) ? cur.pass_legal != 0 : cur.legal.test(a));
-        if (!legal) { *bad = k; break; }
-        const LineHist<G::W> lh = { hist, k };              // the positions before `cur`; next() adds `cur` and the new one
+        if (!legal) { bad[i] = k; break; }
+        const LineHist<G::W> lh = { h, k };                 // the positions before `cur`; next() adds `cur` and the new one
         G::next(cur, a, lh, nx);
         for (int w = 0; w < G::W; ++w) {
-            hist[(size_t)k * 2 * G::W + w] = cur.b[0].word(w);
-            hist[(size_t)k * 2 * G::W + G::W + w] = cur.b[1].word(w);
+            h[(size_t)k * 2 * G::W + w] = cur.b[0].word(w);
+            h[(size_t)k * 2 * G::W + G::W + w] = cur.b[1].word(w);
         }
         cur = nx;
+    }
+}
+
+void env_launch_lines(int game, int n_lines, const long long* off, const int* actions, PosRec* rec, u64* hist, int* bad,
+                      cudaStream_t s) {
+    const int grid = ceil_div(n_lines, 128);
+    switch (game) {
+    case SPRL_GAME_OTHELLO: k_env_lines<Othello><<<grid, 128, 0, s>>>(n_lines, off, actions, rec, hist, bad); break;
+    case SPRL_GAME_C4: k_env_lines<ConnectFour><<<grid, 128, 0, s>>>(n_lines, off, actions, rec, hist, bad); break;
+    case SPRL_GAME_GO7: k_env_lines<Go<7>><<<grid, 128, 0, s>>>(n_lines, off, actions, rec, hist, bad); break;
+    case SPRL_GAME_GO9: k_env_lines<Go<9>><<<grid, 128, 0, s>>>(n_lines, off, actions, rec, hist, bad); break;
+    default: break;
     }
 }
 
@@ -406,10 +391,13 @@ static int env_line_impl(int32_t n_actions, const int32_t* h_actions, int8_t* h_
                          int8_t* h_winner, int8_t* h_mask) {
     if (n_actions > G::MAX_PLIES) return fail(SPRL_E_INVALID, "a line of %d actions is longer than a game (%d plies)", n_actions, G::MAX_PLIES);
     const size_t n = (size_t)n_actions + 1;
-    DeviceBuf<int> dact, dbad; DeviceBuf<PosRec> drec; DeviceBuf<u64> dhist;
+    const long long off[2] = { 0, n_actions };
+    DeviceBuf<int> dact, dbad; DeviceBuf<PosRec> drec; DeviceBuf<u64> dhist; DeviceBuf<long long> doff;
     SPRL_CUDA(dact.alloc(n)); SPRL_CUDA(dbad.alloc(1)); SPRL_CUDA(drec.alloc(n)); SPRL_CUDA(dhist.alloc(n * 2 * G::W));
+    SPRL_CUDA(doff.alloc(2));
+    SPRL_CUDA(cudaMemcpy(doff.p, off, sizeof(off), cudaMemcpyHostToDevice));
     if (n_actions) SPRL_CUDA(cudaMemcpy(dact.p, h_actions, (size_t)n_actions * 4, cudaMemcpyHostToDevice));
-    k_env_line<G><<<1, 32>>>(n_actions, dact.p, drec.p, dhist.p, dbad.p);
+    k_env_lines<G><<<1, 32>>>(1, doff.p, dact.p, drec.p, dhist.p, dbad.p);
     SPRL_CUDA(cudaGetLastError());
     int bad = -1;
     SPRL_CUDA(cudaMemcpy(&bad, dbad.p, 4, cudaMemcpyDeviceToHost));

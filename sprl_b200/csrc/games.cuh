@@ -575,4 +575,36 @@ __host__ __device__ inline int action_slot(const typename G::P& p, int action) {
     return (G::HAS_PASS && action == G::CELLS) ? p.legal.count() : p.legal.rank(action);
 }
 
+// ---- compact position record: exchanged with the host (env.cu) and the opening table of the engine (search.cu) ----
+struct alignas(16) PosRec {
+    u64 b[4];       // b0 words, then b1 words (W each; unused = 0)
+    u64 legal[2];
+    int action;     // action | depth << 8 of the position (rollouts: the action taken from it)
+    unsigned char player, pass_legal, terminal, winner;
+    u32 parent;     // perft: index of the parent in the previous level
+    u32 pad;
+};
+
+template <class G>
+__host__ __device__ inline void pos_to_rec(const typename G::P& p, PosRec& r) {
+    for (int i = 0; i < 2; ++i) {
+        r.b[i] = i < G::W ? p.b[0].word(i) : 0;
+        r.b[2 + i] = i < G::W ? p.b[1].word(i) : 0;
+        r.legal[i] = i < G::W ? p.legal.word(i) : 0;
+    }
+    r.player = p.player; r.pass_legal = p.pass_legal; r.terminal = p.terminal; r.winner = p.winner;
+    r.action = p.action | (p.depth << 8);   // perft keeps action/depth here; rollouts overwrite
+    r.parent = 0; r.pad = 0;
+}
+template <class G>
+__host__ __device__ inline void rec_to_pos(const PosRec& r, typename G::P& p) {
+    for (int i = 0; i < G::W; ++i) {
+        p.b[0].set_word(i, r.b[i]);
+        p.b[1].set_word(i, r.b[2 + i]);
+        p.legal.set_word(i, r.legal[i]);
+    }
+    p.player = r.player; p.pass_legal = r.pass_legal; p.terminal = r.terminal; p.winner = r.winner;
+    p.action = (unsigned char)(r.action & 0xff); p.depth = (unsigned short)(r.action >> 8);
+}
+
 }  // namespace sprl

@@ -315,16 +315,43 @@ struct TreeWarp {
         return true;
     }
 
+    // ---- the game starts from its opening line, as if the caller had advanced a fresh tree through it: the line's
+    //      positions become the game's recorded history (later network inputs, samples, superko), the position it ends in
+    //      becomes the root.  Returns the line's length. ----
+    __device__ int open_line(long long n_lines, P& pos) {
+        const unsigned long long t = MATCH ? st.game_id / 2 : st.game_id;     // match play: both colour assignments of a line
+        const int line = (int)(t % (unsigned long long)n_lines);
+        const int a0 = (int)p.iter->open_off[line];
+        const int len = (int)p.iter->open_off[line + 1] - a0;
+        const PosRec* r = p.iter->open_rec + a0 + line;
+        unsigned long long* rb = p.rec_board + (size_t)st.game_index * p.max_moves * 2 * W;
+        unsigned char* rp = p.rec_player + (size_t)st.game_index * p.max_moves;
+        for (int k = lane; k < len; k += 32) {
+            for (int w = 0; w < W; ++w) { rb[k * 2 * W + w] = r[k].b[w]; rb[k * 2 * W + W + w] = r[k].b[2 + w]; }
+            rp[k] = r[k].player;
+        }
+        rec_to_pos<G>(r[len], pos);
+        return len;
+    }
+
     __device__ void init_game() {
         st.game_id = p.iter->first_game + (unsigned long long)st.game_index * p.iter->game_stride;
         rng.game = st.game_id; rng.ctr = 0;
         st.slab = 0; slab = slab_ptr(0);
         st.traversals = 0; st.move_count = 0; st.n_queued = 0;
-        P start;
-        G::start(start);
+        const long long n_lines = p.iter->n_lines;
         H h;
         if (lane == 0) slab[0] = make_uint4(0u, 0u, 0u, 0u);
-        write_node(slab, ROOT_UNIT, start, 0u, 0u, h);
+        if (n_lines > 0) {
+            P pos;
+            st.move_count = open_line(n_lines, pos);
+            write_node(slab, ROOT_UNIT, pos, 0u, 0u, h);
+        } else {
+            P start;
+            G::start(start);
+            write_node(slab, ROOT_UNIT, start, 0u, 0u, h);
+        }
+        if (lane == 0) p.rec_open[st.game_index] = st.move_count;
         st.n_units = ROOT_UNIT + HDR + META_NLEGAL(h.meta);
         __syncwarp();
     }
@@ -869,7 +896,7 @@ struct TreeWarp {
         if (META_TERMINAL(rmeta)) {
             // game over: the outcome of every recorded move is filled in by the sample writer
             if (lane == 0 && record) {
-                p.rec_moves[st.game_index] = st.move_count;
+                p.rec_moves[st.game_index] = st.move_count - p.rec_open[st.game_index];
                 p.rec_winner[st.game_index] = (unsigned char)META_WINNER(rmeta);
                 p.rec_draws[st.game_index] = rng.ctr;
             }
@@ -894,7 +921,7 @@ struct TreeWarp {
         float sum = 0.0f;
         for (int k = 0; k < n; ++k) sum += sm.pol[legal_action<G>(pos, k)];
         float inv = 1.0f / sum;
-        const float ex = st.move_count < 15 ? 0.98f : 10.0f;       // constants.hpp:8-10
+        const float ex = st.move_count - p.rec_open[st.game_index] < 15 ? 0.98f : 10.0f;   // constants.hpp:8-10; searched moves
         __syncwarp();
         for (int base = 0; base < n; base += 32) {
             int k = base + lane;
@@ -992,7 +1019,7 @@ struct TreeWarp {
         const u32 rmeta = *HL<W>::meta_ptr(slab + ROOT_UNIT);
         if (META_TERMINAL(rmeta)) {
             if (lane == 0) {
-                p.rec_moves[st.game_index] = st.move_count;
+                p.rec_moves[st.game_index] = st.move_count - p.rec_open[st.game_index];
                 p.rec_winner[st.game_index] = (unsigned char)META_WINNER(rmeta);
                 p.rec_draws[st.game_index] = rng.ctr;
             }
@@ -1087,6 +1114,7 @@ __global__ void __launch_bounds__(32) k_match_begin(EngineParams p, MatchParams 
     const int pair = blockIdx.x, lane = threadIdx.x;
     if (pair >= m.n_pairs) return;
     unsigned long long game_id = 0;
+    u32 player = 0;
     for (int k = 0; k < 2; ++k) {
         TreeWarp<G, true> t(p, k * m.n_pairs + pair, lane, scratch, &p.iter->agent[k], m.n_pairs);
         t.st.game_index = pair;
@@ -1094,10 +1122,11 @@ __global__ void __launch_bounds__(32) k_match_begin(EngineParams p, MatchParams 
         if (t.st.game_index < p.iter->num_games) { t.st.status = ST_PLAYING; t.init_game(); }
         else t.st.status = ST_DONE;
         game_id = t.st.game_id;
+        player = META_PLAYER(*HL<G::W>::meta_ptr(t.slab + ROOT_UNIT));
         t.save();
     }
     __syncwarp();
-    if (lane == 0) p.trees[pair].pad = (u32)(game_id & 1ULL);     // Player ZERO moves first
+    if (lane == 0) p.trees[pair].pad = player ^ (u32)(game_id & 1ULL);     // the side to move (ZERO, unless an opening line says otherwise)
 }
 
 template <class G>
@@ -1207,13 +1236,13 @@ __global__ void k_emit(EngineParams p, long long g0, const long long* __restrict
                        float* __restrict__ states, float* __restrict__ dists, float* __restrict__ outcomes) {
     constexpr int W = G::W, PLANES = 2 * G::HISTORY + 1, ROW = PLANES * G::CELLS;
     const long long g = g0 + blockIdx.x;    // grid = (games of the range, max_moves)
-    const int m = (int)blockIdx.y;
-    if (m >= p.rec_moves[g]) return;
+    if ((int)blockIdx.y >= p.rec_moves[g]) return;
+    const int m = p.rec_open[g] + (int)blockIdx.y;     // searched move blockIdx.y; the opening's plies are history only
     const size_t ri = (size_t)g * p.max_moves + m;
     const int player = p.rec_player[ri];
     const unsigned char wn = p.rec_winner[g];
     const float outcome = (wn == WINNER_NONE) ? 0.0f : ((int)wn - 1 == player ? 1.0f : -1.0f);
-    const long long row0 = game_row0[g] + (long long)m * S;
+    const long long row0 = game_row0[g] + (long long)blockIdx.y * S;
     // one thread per (symmetry, cell): the source cell is found once and serves every plane; a warp's
     // stores to a plane are contiguous
     for (int idx = threadIdx.x; idx < S * G::CELLS; idx += blockDim.x) {

@@ -86,6 +86,13 @@ struct IterParams {
     int step_sims;
     int step_single;                 // one searchAndGetLeaves batch per launch, whatever the evaluator (sprl_search_batch)
     AgentCfg agent[2];               // match play: the two sides
+    // opening lines (sprl_set_openings; n_lines = 0: every game starts at the start position).  Stream id t plays line
+    // t % n_lines (match play: (t / 2) % n_lines, so that both colour assignments play each line).  Line i has
+    // open_off[i+1] - open_off[i] actions; its positions are open_rec[open_off[i] + i ..  open_off[i+1] + i]: the position
+    // each of its actions is played in, then the position it ends in.  Read by init_game whenever a slot starts a game.
+    long long n_lines;
+    const long long* open_off;       // [n_lines + 1]
+    const PosRec* open_rec;          // [open_off[n_lines] + n_lines]
 };
 
 struct EngineParams {
@@ -120,7 +127,8 @@ struct EngineParams {
     unsigned long long* rec_board;  // [..][2W]
     unsigned char* rec_player;      // [..]
     float* rec_pdf;                 // [..][A]
-    int* rec_moves;                 // [num_games]
+    int* rec_moves;                 // [num_games] searched moves (the opening's plies excluded) of a finished game, 0 before
+    int* rec_open;                  // [num_games] plies of the game's opening line: its searched moves are recorded from there on
     unsigned char* rec_winner;      // [num_games]
     unsigned long long* rec_draws;  // [num_games]
     // optional per-move search statistics (parity tests)

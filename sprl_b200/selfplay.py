@@ -130,6 +130,17 @@ class Engine:
     def set_game_stride(self, stride):
         capi.check(self.lib.sprl_set_game_stride(self.handle, stride))
 
+    def set_openings(self, lines):
+        """Opening lines (sequences of actions from the start position) for the games and trees that the next
+        run_iteration / run_match / begin_trees starts: stream id t starts from line t % len(lines), a match game from
+        line (t // 2) % len(lines) with both colour assignments.  Samples and move records cover the searched moves only.
+        An empty sequence turns openings off (sprl_set_openings)."""
+        lines = [np.asarray(line, np.int64).reshape(-1) for line in lines]
+        offsets = np.zeros(len(lines) + 1, np.int64)
+        offsets[1:] = np.cumsum([len(line) for line in lines])
+        actions = np.ascontiguousarray(np.concatenate(lines) if lines else np.zeros(0), np.int32)
+        capi.check(self.lib.sprl_set_openings(self.handle, len(lines), _ptr(offsets), _ptr(actions)))
+
     @property
     def eval_batch(self):
         return self.lib.sprl_eval_batch(self.handle)
